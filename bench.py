@@ -5,6 +5,7 @@
                                                              # torch.distributed.run: CFG halves x frame shards)
     python bench.py --impl reference --steps K --warmup W    # the UNMODIFIED reference forward on the host CPU cores
     python bench.py --workload interp|vsr|encoders           # BASELINE configs 4 / 5 and the once-per-video stages
+    python bench.py ... --dump-outputs DIR                   # also write the last timed step's outputs as DIR/*.npy
 
 A "step" is one CFG denoising step of VideoGenPipeline's loop (pipeline_videogen.py:664-689): the UNet forward on
 [2,4,16,40,64] (uncond + cond), the guidance combine and the DDIM update.  Weights are deterministic random-init of
@@ -103,6 +104,25 @@ class ClockSampler:
                 "samples": len(sm)}
 
 
+DUMP_BYTES = 64_000_000
+
+
+def dump_outputs(directory, arrays):
+    """--dump-outputs: write what the timed path returned in its last step, one float32 DIR/<name>.npy per array.  The
+    inputs are seeded, so two builds run with the same arguments can be compared output for output.  The dump stays
+    within 64 MB: an array larger than its share is written as <name>_sample.npy, a fixed seeded choice of its elements
+    (the same positions for the same shape)."""
+    import numpy as np
+    os.makedirs(directory, exist_ok=True)
+    share = (DUMP_BYTES // len(arrays) - 256) // 4          # elements per array; 256 bytes for the .npy header
+    for name, t in arrays.items():
+        a = t.detach().cpu().float()
+        if a.numel() > share:
+            idx = torch.randperm(a.numel(), generator=torch.Generator().manual_seed(0))[:share].sort().values
+            a, name = a.reshape(-1)[idx], f"{name}_sample"
+        np.save(os.path.join(directory, f"{name}.npy"), a.numpy())
+
+
 # ----------------------------------------------------------------------------------------------- CPU legs
 CONFIG = {"workload": WORKLOAD, "weights": "random-init (seeded), 909.1 M params", "timesteps": "DDIM, 50 steps"}
 
@@ -168,7 +188,10 @@ def run_reference(args):
             frames = f
     for _ in range(args.warmup):
         timed_forward(fwd, frames)
-    times = [timed_forward(fwd, frames)[0] for _ in range(args.steps)]
+    times = []
+    for _ in range(args.steps):
+        dt, out = timed_forward(fwd, frames)
+        times.append(dt)
     step_s = sum(times) / len(times)
     frac = frames / FRAMES
     value = frac / step_s
@@ -181,6 +204,8 @@ def run_reference(args):
             "cpu_baseline": {"value": value, "unit": "steps/s", "cores": threads, "kind": kind, "sample": sample},
             "e2e": {"value": value, "unit": "steps/s", "h2d_bytes_per_step": 0, "d2h_bytes_per_step": 0},
             "gpu_launches": 0}
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"noise_pred": out})
     print(json.dumps(line), flush=True)
 
 
@@ -298,6 +323,7 @@ def run_b200(args):
             x = one_step(x, timesteps[i % len(timesteps)])
         ev1.record()
         barrier()
+    dump = {"latents": x.cpu()} if args.dump_outputs else None
     ms = ev0.elapsed_time(ev1)
     if world > 1:
         tmax = torch.tensor([ms], device=dev)
@@ -426,6 +452,8 @@ def run_b200(args):
                 "clocks": clocks.summary(),
                 "e2e": {"value": e2e_value, "unit": "steps/s", "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": d2h},
                 "gpu_launches": gpu_launches, "roofline": roofline, "cpu_baseline": cpu, "kernels": kernels}
+        if dump is not None:
+            dump_outputs(args.dump_outputs, dump)
         print(json.dumps(line), flush=True)
     if world > 1:
         torch.cuda.synchronize()
@@ -543,6 +571,7 @@ def run_interp(args):
             x = one_step(x, cnd, txt, i)
         ev1.record()
         barrier()
+    dump = {"latents": x.cpu()} if args.dump_outputs else None
     ms = ev0.elapsed_time(ev1)
     if world > 1:
         tmax = torch.tensor([ms], device=dev)
@@ -637,6 +666,8 @@ def run_interp(args):
                         "h2d_bytes_per_step": (xh[0].numel() + ch.numel() + th.numel()) * 4,
                         "d2h_bytes_per_step": xh[0].numel() * 4},
                 "gpu_launches": per_step * args.steps, "roofline": roofline, "cpu_baseline": cpu, "kernels": kernels}
+        if dump is not None:
+            dump_outputs(args.dump_outputs, dump)
         print(json.dumps(line), flush=True)
     if world > 1:
         torch.cuda.synchronize()
@@ -761,6 +792,7 @@ def run_vsr(args):
             x = one_step(x, lowd, txt, i)
         ev1.record()
         barrier()
+    dump = {"latents": x.cpu()} if args.dump_outputs else None
     ms = ev0.elapsed_time(ev1)
     if world > 1:
         tmax = torch.tensor([ms], device=dev)
@@ -865,6 +897,8 @@ def run_vsr(args):
                     "h2d_bytes_per_step": (xh[0].numel() + lh.numel() + th.numel()) * 4,
                     "d2h_bytes_per_step": xh[0].numel() * 4},
             "gpu_launches": per_step * args.steps, "roofline": roofline, "cpu_baseline": cpu, "kernels": kernels}
+    if dump is not None:
+        dump_outputs(args.dump_outputs, dump)
     print(json.dumps(line), flush=True)
     if world > 1:
         torch.cuda.synchronize()
@@ -912,9 +946,10 @@ def run_encoders(args):
         torch.cuda.synchronize()
         ev0.record()
         for _ in range(args.steps):
-            one_step(latd, idsd)
+            video, emb = one_step(latd, idsd)
         ev1.record()
         torch.cuda.synchronize()
+    dump = {"video": video.cpu(), "text_embedding": emb.cpu()} if args.dump_outputs else None
     ms_per_step = ev0.elapsed_time(ev1) / args.steps
     lh, ih = lat.clone().pin_memory(), ids.clone().pin_memory()
     vid_h = torch.empty((FRAMES, 8 * LAT_H, 8 * LAT_W, 3), dtype=torch.uint8).pin_memory()
@@ -978,6 +1013,8 @@ def run_encoders(args):
             "e2e": {"value": args.steps / e2e_s, "unit": "videos/s", "h2d_bytes_per_step": lh.numel() * 4 + ih.numel() * 8,
                     "d2h_bytes_per_step": vid_h.numel() + emb_h.numel() * 4},
             "gpu_launches": per_step * args.steps, "roofline": roofline, "cpu_baseline": cpu, "kernels": kernels}
+    if dump is not None:
+        dump_outputs(args.dump_outputs, dump)
     print(json.dumps(line), flush=True)
 
 
@@ -993,7 +1030,13 @@ def main():
     ap.add_argument("--vsr-height", type=int, default=320)
     ap.add_argument("--vsr-width", type=int, default=512)
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one as DIR/<name>.npy (float32)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and int(os.environ.get("WORLD_SIZE", "1")) > 1:
+        ap.error("--dump-outputs runs in one process (each rank of a sharded run holds only its frames)")
     if args.impl == "reference":
         run_reference(args)
     elif args.workload == "interp":

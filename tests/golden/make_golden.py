@@ -13,6 +13,7 @@ fp32 and stores inputs, a few intermediate activations (forward hooks) and the o
 Nothing under tests/, bench.py or smoke() reads /root/reference at run time; they read the
 .pt files written here.
 """
+import hashlib
 import os
 import sys
 import time
@@ -40,6 +41,9 @@ TAPS = {
     "down0_attn0": "down_blocks.0.attentions.0",
     "mid": "mid_block",
 }
+# kept under 1 MB: taps at every 16th channel instead of every 8th, the text embedding as the digest of its bytes
+# (tests/conftest.py:load_golden draws it again from the inputs seed)
+LEAN = {"b2_f16_8x8"}
 
 
 def main():
@@ -51,12 +55,13 @@ def main():
     mods = dict(ref.named_modules())
     for name, (b, f, h, w, t) in CASES.items():
         sample, _, text = synthetic_inputs(b, f, h, w, seed=1)
+        stride = 16 if name in LEAN else 8
         got = {}
         hooks = []
         for tap, modname in TAPS.items():
             def hook(_m, _i, out, tap=tap):
                 out = out.sample if hasattr(out, "sample") else out
-                got[tap] = out.detach()[:, ::8].contiguous().clone()   # every 8th channel keeps the fixture small
+                got[tap] = out.detach()[:, ::stride].contiguous().clone()   # a channel subset keeps the fixture small
             hooks.append(mods[modname].register_forward_hook(hook))
         t0 = time.time()
         with torch.no_grad():
@@ -66,6 +71,8 @@ def main():
             hk.remove()
         blob = {"sample": sample, "timestep": t, "text": text, "out": out, "taps": got,
                 "weights_seed": 0, "inputs_seed": 1, "shape": (b, f, h, w)}
+        if name in LEAN:
+            blob["text_sha256"] = hashlib.sha256(blob.pop("text").numpy().tobytes()).hexdigest()
         torch.save(blob, os.path.join(HERE, f"{name}.pt"))
         print(f"{name}: out std {out.std():.4f} in {dt:.1f}s -> {name}.pt")
     # one timestep passed as a [B] tensor with different values per batch item

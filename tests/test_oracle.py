@@ -18,7 +18,9 @@ def test_oracle_matches_reference_forward(name, synthetic_sd):
     assert rel_l2(out, g["out"]) < 2e-5
     assert (out - g["out"]).abs().max() < 2e-4
     for k, ref in g["taps"].items():
-        assert rel_l2(taps[k][:, ::8], ref) < 2e-5, k
+        got = taps[k][:, ::taps[k].shape[1] // ref.shape[1]]          # the golden keeps every 8th or 16th channel
+        assert got.shape == ref.shape, k
+        assert rel_l2(got, ref) < 2e-5, k
 
 
 def test_synthetic_weights_are_reproducible(synthetic_sd):
