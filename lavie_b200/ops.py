@@ -738,6 +738,22 @@ def softmax_rows_(s: torch.Tensor, scale: float) -> torch.Tensor:
     return s
 
 
+def pointwise_conv_nchw(x: torch.Tensor, w: torch.Tensor, bias: torch.Tensor, scale: float = 1.0) -> torch.Tensor:
+    """1x1 conv on an fp32 NCHW map: x [N, Cin, h, w], w fp32 [Cout, Cin], bias fp32 [Cout] -> fp32 [N, Cout, h, w]
+    = bias + w @ (scale * x) per pixel (AutoencoderKL.post_quant_conv with decode_latents' scaling folded in)."""
+    lib = _lib.load()
+    assert x.dtype == F32 and x.is_contiguous() and x.dim() == 4
+    N, Cin, h, wd = x.shape
+    Cout = w.shape[0]
+    assert w.dtype == F32 and w.is_contiguous() and tuple(w.shape) == (Cout, Cin)
+    assert bias.dtype == F32 and bias.is_contiguous() and bias.numel() == Cout
+    out = torch.empty((N, Cout, h, wd), dtype=F32, device=x.device)
+    with _Launch("lavie_pointwise_conv_nchw_f32"):
+        check(lib.lavie_pointwise_conv_nchw_f32(x.data_ptr(), w.data_ptr(), bias.data_ptr(), float(scale), N, Cin, Cout,
+                                                h * wd, out.data_ptr(), _stream()), "lavie_pointwise_conv_nchw_f32")
+    return out
+
+
 def image_to_uint8(y: torch.Tensor) -> torch.Tensor:
     """y bf16 [pixels, >= 4] channels-last (columns 0..2 = RGB in [-1, 1]) -> uint8 [pixels, 3]."""
     lib = _lib.load()

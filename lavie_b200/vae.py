@@ -18,7 +18,7 @@ from typing import Dict, Tuple
 import torch
 from torch import nn
 
-from . import _lib, ops
+from . import ops
 from .packing import pack_conv1x1, pack_conv3x3, pack_upsample_conv3x3
 from .synthetic import _gen
 
@@ -214,15 +214,10 @@ class VAEDecoder(nn.Module):
         if z.dim() != 4 or z.shape[1] != 4:
             raise ValueError(f"z must be [N,4,h,w], got {tuple(z.shape)}")
         P = self._packed or self._pack()
-        lib = _lib.load()
         dev = self.device
         N, _, h, w = z.shape
         zin = z.to(device=dev, dtype=F32).contiguous()
-        zq = torch.empty_like(zin)
-        with ops._Launch("lavie_pointwise_conv_nchw_f32"):
-            ops.check(lib.lavie_pointwise_conv_nchw_f32(zin.data_ptr(), P["pq"][0].data_ptr(), P["pq"][1].data_ptr(),
-                                                        float(scale), N, 4, 4, h * w, zq.data_ptr(), ops._stream()),
-                      "lavie_pointwise_conv_nchw_f32")
+        zq = ops.pointwise_conv_nchw(zin, P["pq"][0], P["pq"][1], scale)
         x = ops.conv_in(zq.reshape(N, 4, 1, h, w), P["conv_in"][0], P["conv_in"][1])
         H, W = h, w
         x = self._resnet("decoder.mid_block.resnets.0", x, N, H, W)

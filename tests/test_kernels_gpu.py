@@ -13,6 +13,16 @@ pytestmark = pytest.mark.gpu
 DEV = "cuda"
 
 
+@pytest.fixture(autouse=True, scope="module")
+def _exact_fp32_references():
+    """The fp32 references (F.conv2d, matmul) run on the GPU: keep TF32 off for cuDNN and cuBLAS, else a reference
+    carries ~bf16-sized error of its own."""
+    saved = torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32
+    torch.backends.cudnn.allow_tf32 = torch.backends.cuda.matmul.allow_tf32 = False
+    yield
+    torch.backends.cudnn.allow_tf32, torch.backends.cuda.matmul.allow_tf32 = saved
+
+
 def _ops():
     from lavie_b200 import ops
     return ops
