@@ -10,7 +10,7 @@ from __future__ import annotations
 
 from dataclasses import dataclass
 from types import SimpleNamespace
-from typing import Dict, List, Optional, Tuple, Union
+from typing import Dict, Optional, Tuple, Union
 
 import torch
 from torch import nn
@@ -95,9 +95,11 @@ def _install(root: nn.Module, path: str, leaf: nn.Module) -> None:
 
 
 class UNet3DConditionModel(nn.Module):
-    """B200-native LaVie base denoiser.  ``use_cuda_graph`` replays the whole step from one captured CUDA graph per
+    """B200-native LaVie base denoiser (and, by ``config.variant``, the interpolation one; the VSR one is the subclass
+    lavie_b200.vsr.UNet3DVSRModel).  ``use_cuda_graph`` replays the whole step from one captured CUDA graph per
     input geometry (the reference launches ~1.9k kernels per step from Python)."""
     _VARIANTS = ("base", "interp")
+    _TAPS = ("emb", "conv_in", "down0_res0", "down0_attn0", "mid", "up_out")     # the oracle's tap points (forward(taps=))
 
     def __init__(self, config: UNetConfig = BASE_CONFIG, use_cuda_graph: bool = True, check_mode: bool = False):
         """``check_mode=True``: the fp32-accumulate check mode of BASELINE's north star (rel-L2 <= 1e-3 vs the reference
@@ -279,14 +281,15 @@ class UNet3DConditionModel(nn.Module):
     # ------------------------------------------------------------------ weight packing (post-load)
     def _pack(self):
         sd = {k: v.detach() for k, v in self.state_dict().items()}
-        missing = [k for k in param_spec(self.cfg) if k not in sd]
+        spec = param_spec(self.cfg)
+        missing = [k for k in spec if k not in sd]
         if missing:
             raise RuntimeError(f"state_dict no longer has the reference layout (first missing key: {missing[0]}); "
                                "wrapped / replaced leaf modules (e.g. un-merged LoRA adapters) are not executed by the "
                                "fused path -- merge them into the base weights first")
         dev = self.device
         if dev.type != "cuda":
-            raise RuntimeError("lavie_b200.UNet3DConditionModel runs on CUDA (sm_100a) only; move it with .to('cuda')")
+            raise RuntimeError(f"lavie_b200.{type(self).__name__} runs on CUDA (sm_100a) only; move it with .to('cuda')")
         heads = self.cfg.heads
         P: Dict[str, object] = {}
 
@@ -298,69 +301,96 @@ class UNet3DConditionModel(nn.Module):
         def pack_conv3x3_(w):            # layout only; precision is decided by K.weight
             return pack_conv3x3(w, dtype=None)
 
-        def pack_conv1x1_(w):
+        def pack_conv1x1_(w):            # 1x1 conv or Linear (the VSR model's proj_in / proj_out)
             return pack_conv1x1(w, dtype=None)
 
         def b16(t):                      # kernel-side weight matrix: bf16 (check mode: an (hi, lo) bf16 pair)
             return K.weight(t, dev)
 
+        # every time_emb_proj in one matrix and every text K/V projection in another, rows in param_spec order
         temb_w, temb_b, temb_slices = [], [], {}
-        kv_w, kv_slices = [], {}
+        kv_w = []
         temb_off = 0
         kv_off = 0
 
-        def pack_resnet(p):
-            nonlocal temb_off
-            r = {"g1": f32(f"{p}.norm1.weight"), "b1": f32(f"{p}.norm1.bias"),
-                 "w1": b16(pack_conv3x3_(sd[f"{p}.conv1.weight"])), "cb1": f32(f"{p}.conv1.bias"),
-                 "g2": f32(f"{p}.norm2.weight"), "b2": f32(f"{p}.norm2.bias"),
-                 "w2": b16(pack_conv3x3_(sd[f"{p}.conv2.weight"])), "cb2": f32(f"{p}.conv2.bias")}
-            cout = sd[f"{p}.conv1.weight"].shape[0]
-            temb_w.append(sd[f"{p}.time_emb_proj.weight"])
-            temb_b.append(sd[f"{p}.time_emb_proj.bias"])
-            temb_slices[p] = (temb_off, cout)
-            temb_off += cout
-            if f"{p}.conv_shortcut.weight" in sd:
-                r["wsc"] = b16(pack_conv1x1_(sd[f"{p}.conv_shortcut.weight"]))
-                r["bsc"] = f32(f"{p}.conv_shortcut.bias")
+        for key, shape in spec.items():
+            if not key.endswith(".conv1.weight"):
+                continue
+            p = key[: -len(".conv1.weight")]
+            r = {"g1": f32(f"{p}.norm1.weight"), "b1": f32(f"{p}.norm1.bias"), "cb1": f32(f"{p}.conv1.bias"),
+                 "g2": f32(f"{p}.norm2.weight"), "b2": f32(f"{p}.norm2.bias"), "cb2": f32(f"{p}.conv2.bias")}
+            if len(shape) == 5:                                   # ResnetBlock3DCNN (vsr/models/resnet.py:220-316)
+                from .vsr import pack_frame_conv
+                r["k"] = shape[2]
+                r["w1"] = b16(pack_frame_conv(sd[f"{p}.conv1.weight"]))
+                r["w2"] = b16(pack_frame_conv(sd[f"{p}.conv2.weight"]))
+            else:                                                 # ResnetBlock3D
+                r["w1"] = b16(pack_conv3x3_(sd[f"{p}.conv1.weight"]))
+                r["w2"] = b16(pack_conv3x3_(sd[f"{p}.conv2.weight"]))
+                if f"{p}.conv_shortcut.weight" in sd:
+                    r["wsc"] = b16(pack_conv1x1_(sd[f"{p}.conv_shortcut.weight"]))
+                    r["bsc"] = f32(f"{p}.conv_shortcut.bias")
+                if "temporal_block" in p:                         # TemporalModule3D builds it with the default eps
+                    r["eps"] = 1e-6
+            if f"{p}.time_emb_proj.weight" in sd:
+                temb_w.append(sd[f"{p}.time_emb_proj.weight"])
+                temb_b.append(sd[f"{p}.time_emb_proj.bias"])
+                temb_slices[p] = (temb_off, shape[0])
+                temb_off += shape[0]
             P[p] = r
 
-        def pack_transformer(p):
-            nonlocal kv_off
+        # the VSR tree names the temporal attention and its LayerNorm attn_temporal / norm_temporal
+        tmp = "temporal" if self.cfg.variant == "vsr" else "temp"
+        for key in spec:
+            if not key.endswith(".proj_in.weight"):
+                continue
+            p = key[: -len(".proj_in.weight")]
             b = f"{p}.transformer_blocks.0"
             C = sd[f"{p}.norm.weight"].shape[0]
             d = C // heads
             hp = heads * head_pitch(d)
-            t = {"C": C, "d": d, "pitch": head_pitch(d), "hp": hp,
+            only_cross = any(self.cfg.only_cross_attention) and self._only_cross_for(p)
+
+            def qkv(a):
+                return b16(torch.cat([pad_heads(sd[f"{b}.{a}.to_{x}.weight"], heads) for x in "qkv"], 0))
+
+            def text_kv(a):              # rows of the one text K/V GEMM; returns their first column
+                nonlocal kv_off
+                kv_w.append(pad_heads(sd[f"{b}.{a}.to_k.weight"], heads))
+                kv_w.append(pad_heads(sd[f"{b}.{a}.to_v.weight"], heads))
+                kv_off += 2 * hp
+                return kv_off - 2 * hp
+
+            t = {"C": C, "d": d, "pitch": head_pitch(d), "hp": hp, "only_cross": only_cross,
                  "gn_g": f32(f"{p}.norm.weight"), "gn_b": f32(f"{p}.norm.bias"),
                  "w_in": b16(pack_conv1x1_(sd[f"{p}.proj_in.weight"])), "b_in": f32(f"{p}.proj_in.bias"),
                  "w_out": b16(pack_conv1x1_(sd[f"{p}.proj_out.weight"])), "b_out": f32(f"{p}.proj_out.bias")}
-            for n in ("norm1", "norm2", "norm_temp", "norm3"):
-                t[f"{n}_g"] = f32(f"{b}.{n}.weight")
-                t[f"{n}_b"] = f32(f"{b}.{n}.bias")
-            for a in ("attn1", "attn_temp"):
-                t[f"{a}_qkv"] = b16(torch.cat([pad_heads(sd[f"{b}.{a}.to_{x}.weight"], heads) for x in "qkv"], 0))
-                t[f"{a}_wo"] = b16(sd[f"{b}.{a}.to_out.0.weight"])
-                t[f"{a}_bo"] = f32(f"{b}.{a}.to_out.0.bias")
+            for n, src in (("norm1", "norm1"), ("norm2", "norm2"), ("norm_temp", f"norm_{tmp}"), ("norm3", "norm3")):
+                t[f"{n}_g"] = f32(f"{b}.{src}.weight")
+                t[f"{n}_b"] = f32(f"{b}.{src}.bias")
+            if only_cross:               # attn1 reads the text (the VSR model's only_cross_attention levels)
+                t["attn1_q"] = b16(pad_heads(sd[f"{b}.attn1.to_q.weight"], heads))
+                t["attn1_kv_off"] = text_kv("attn1")
+            else:
+                t["attn1_qkv"] = qkv("attn1")
+            t["attn_temp_qkv"] = qkv(f"attn_{tmp}")
+            for a, src in (("attn1", "attn1"), ("attn2", "attn2"), ("attn_temp", f"attn_{tmp}")):
+                t[f"{a}_wo"] = b16(sd[f"{b}.{src}.to_out.0.weight"])
+                t[f"{a}_bo"] = f32(f"{b}.{src}.to_out.0.bias")
             t["attn2_q"] = b16(pad_heads(sd[f"{b}.attn2.to_q.weight"], heads))
-            t["attn2_wo"] = b16(sd[f"{b}.attn2.to_out.0.weight"])
-            t["attn2_bo"] = f32(f"{b}.attn2.to_out.0.bias")
-            kv_w.append(pad_heads(sd[f"{b}.attn2.to_k.weight"], heads))
-            kv_w.append(pad_heads(sd[f"{b}.attn2.to_v.weight"], heads))
-            t["kv_off"] = kv_off
-            kv_off += 2 * hp
+            t["kv_off"] = text_kv("attn2")
             wi, bi = interleave_geglu(sd[f"{b}.ff.net.0.proj.weight"], sd[f"{b}.ff.net.0.proj.bias"])
             t["ff1_w"], t["ff1_b"] = b16(wi), bi.to(device=dev, dtype=F32).contiguous()
             t["ff2_w"], t["ff2_b"] = b16(sd[f"{b}.ff.net.2.weight"]), f32(f"{b}.ff.net.2.bias")
-            if self.cfg.variant == "base":      # the interpolation model's temporal attention has neither (SURVEY 2 #13)
-                t["rel_emb"] = f32(f"{b}.attn_temp.time_rel_pos_bias.relative_attention_bias.weight")
-                t["freqs"] = f32(f"{b}.attn_temp.rotary_emb.freqs")
+            if self.cfg.variant != "interp":    # the interpolation model's temporal attention has neither (SURVEY 2 #13)
+                t["rel_emb"] = f32(f"{b}.attn_{tmp}.time_rel_pos_bias.relative_attention_bias.weight")
+                t["freqs"] = f32(f"{b}.attn_{tmp}.rotary_emb.freqs")
             P[p] = t
 
-        for key in self._resnet_prefixes():
-            pack_resnet(key)
-        for key in self._transformer_prefixes():
-            pack_transformer(key)
+        for key in spec:
+            if key.endswith(".shift_conv.weight"):                # TemporalModule3D's 1x1 conv
+                p = key[: -len(".shift_conv.weight")]
+                P[f"{p}.shift_conv"] = (b16(pack_conv1x1_(sd[key])), f32(f"{p}.shift_conv.bias"))
         for i in range(len(self.cfg.block_out_channels) - 1):
             P[f"down_blocks.{i}.downsamplers.0.conv"] = (
                 b16(pack_conv3x3_(sd[f"down_blocks.{i}.downsamplers.0.conv.weight"])),
@@ -388,19 +418,14 @@ class UNet3DConditionModel(nn.Module):
         P["norm_out"] = (f32("conv_norm_out.weight"), f32("conv_norm_out.bias"))
         P["time1"] = (K.weight_small(sd["time_embedding.linear_1.weight"], dev), f32("time_embedding.linear_1.bias"))
         P["time2"] = (K.weight_small(sd["time_embedding.linear_2.weight"], dev), f32("time_embedding.linear_2.bias"))
+        if self.cfg.num_class_embeds:
+            P["class_emb"] = f32("class_embedding.weight")
         P["temb_w"] = K.weight_small(torch.cat(temb_w, 0), dev)
         P["temb_b"] = torch.cat(temb_b, 0).to(device=dev, dtype=F32).contiguous()
         P["temb_slices"] = temb_slices
         P["kv_w"] = b16(torch.cat(kv_w, 0))
         self._packed = P
         return P
-
-    def _resnet_prefixes(self) -> List[str]:
-        keys = [k[: -len(".conv1.weight")] for k in param_spec(self.cfg) if k.endswith(".conv1.weight")]
-        return keys
-
-    def _transformer_prefixes(self) -> List[str]:
-        return [k[: -len(".proj_in.weight")] for k in param_spec(self.cfg) if k.endswith(".proj_in.weight")]
 
     def _frame_tables(self, prefix: str, frames: int):
         key = (prefix, frames)
@@ -432,18 +457,26 @@ class UNet3DConditionModel(nn.Module):
         return K.conv3x3(h, NF, H, W, r["w2"], bias=r["cb2"], residual=sc, stats=True)
 
     def _transformer(self, p, x, kv_all, B, Fr, H, W, text_len):
-        """Transformer3DModel.forward + BasicTransformerBlock.forward (attention.py:358-407, 511-560)."""
+        """Transformer3DModel.forward + BasicTransformerBlock.forward (attention.py:358-407, 511-560; VSR tree:
+        vsr/models/attention.py:386-438, 556-593)."""
         K = self._k
         t = self._packed[p]
         heads, d, pitch, hp = self.cfg.heads, t["d"], t["pitch"], t["hp"]
         NF, HW = B * Fr, H * W
         interp = self.cfg.variant == "interp"
+        if self.cfg.variant == "vsr":          # the VSR transformer runs a temporal (3,1,1) ResNet on its input first
+            x = self._resnet_cnn(f"{p}.resblock_temporal", x, None, B, Fr, HW)
         h = K.groupnorm(x, NF, HW, t["gn_g"], t["gn_b"], 1e-6, silu=False)            # per-frame GN (4-D input)
         tok = K.gemm(h, t["w_in"], bias=t["b_in"])
         # spatial self-attention; interpolation model: SparseCausalAttention, the keys of frame f are those of frame 0
         # and of frame f-1 (interpolation/models/attention.py:611-664) -- two key segments, never concatenated
         n = K.layernorm(tok, t["norm1_g"], t["norm1_b"])
-        if interp and self._shard is not None:
+        if t["only_cross"]:                    # attn1 reads the text (the VSR model's only_cross_attention levels)
+            q = K.gemm(n, t["attn1_q"])
+            ko = t["attn1_kv_off"]
+            a = K.attention(q, K.cols(kv_all, ko, ko + hp), K.cols(kv_all, ko + hp, ko + 2 * hp), NF, heads, HW, text_len,
+                            d, pitch, kv_batch_div=Fr)
+        elif interp and self._shard is not None:
             # frame-sharded SparseCausal attention: q|k|v of the local frames land behind two halo frames that the first
             # rank (frame 0 of the video) and the left neighbour (its last frame) fill over NVLink
             assert B == 1, "frame sharding runs one CFG half per rank"
@@ -549,11 +582,12 @@ class UNet3DConditionModel(nn.Module):
         return K.gemm(tok, t["w_out"], bias=t["b_out"], residual=x, stats=True)
 
     def _step(self, sample: torch.Tensor, t: torch.Tensor, text: torch.Tensor, taps: Optional[dict] = None,
-              input_scale: Optional[torch.Tensor] = None, kv_all: Optional[torch.Tensor] = None):
-        """One denoiser evaluation.  sample fp32 [B,C,F,H,W], t fp32 [B], text [B*L, ctx] (bf16; fp32 in check mode)
-        -> fp32 [B,Co,F,H,W].  ``kv_all``: the text K/V projections when the caller already holds them (graph path: they
-        are computed once per prompt, not once per step -- the reference re-projects them in every attn2 call,
-        attention.py:364)."""
+              input_scale: Optional[torch.Tensor] = None, kv_all: Optional[torch.Tensor] = None,
+              labels: Optional[torch.Tensor] = None):
+        """One denoiser evaluation.  sample fp32 [B,C,F,H,W] (VSR: latent | low-res frames), t fp32 [B], text [B*L, ctx]
+        (bf16; fp32 in check mode), labels int64 [B] (VSR noise level) -> fp32 [B,Co,F,H,W].  ``kv_all``: the text K/V
+        projections when the caller already holds them (graph path: they are computed once per prompt, not once per
+        step -- the reference re-projects them in every attn2 call, attention.py:364)."""
         K = self._k
         P = self._packed
         cfg = self.cfg
@@ -572,17 +606,19 @@ class UNet3DConditionModel(nn.Module):
             self._peer_ctx(B * f_total * (H * W // P_) * boc[0] * 2, halo, f_off if self._frame_counts else -1)
 
         def tap(name, x, C, h, w):
-            if taps is not None:
+            if taps is not None and name in self._TAPS:
                 taps[name] = K.to_float(x).reshape(B, Fr, h, w, C).permute(0, 4, 1, 2, 3).contiguous()
 
         # time embedding (unet.py:428-434) and all 22 time_emb_proj (resnet.py:187) in three small launches
         temb = K.timestep_embedding(t, boc[0])
         h1 = K.linear_smallm(temb, P["time1"][0], P["time1"][1], silu_out=True)
         emb = K.linear_smallm(h1, P["time2"][0], P["time2"][1])
+        if cfg.num_class_embeds:               # + the noise-level class embedding (vsr/models/unet.py:494-507)
+            ops.embedding_add(emb, P["class_emb"], labels)
         temb_all = K.linear_smallm(emb, P["temb_w"], P["temb_b"], silu_in=True)
-        if taps is not None:
+        if taps is not None and "emb" in self._TAPS:
             taps["emb"] = emb.clone()
-        # all 16 cross-attention K/V projections of the text in one GEMM
+        # every K/V projection of the text in one GEMM (the base model's 16 cross-attentions)
         if kv_all is None:
             kv_all = K.gemm(text, P["kv_w"])
 
@@ -591,7 +627,7 @@ class UNet3DConditionModel(nn.Module):
         else:
             x = K.conv_in(sample, P["conv_in"][0], P["conv_in"][1], input_scale)
         tap("conv_in", x, boc[0], H, W)
-        skips = [(x, boc[0])]
+        skips = [x]
         h, w = H, W
         for i, kind in enumerate(cfg.down_block_types):
             for j in range(cfg.layers_per_block):
@@ -602,25 +638,33 @@ class UNet3DConditionModel(nn.Module):
                     x = self._transformer(f"down_blocks.{i}.attentions.{j}", x, kv_all, B, Fr, h, w, text_len)
                     if i == 0 and j == 0:
                         tap("down0_attn0", x, boc[0], h, w)
-                skips.append((x, boc[i]))
+                skips.append(x)
             if i != len(boc) - 1:
                 wd, bd = P[f"down_blocks.{i}.downsamplers.0.conv"]
                 x = K.conv3x3(x, B * Fr, h, w, wd, stride=2, bias=bd, stats=True)
                 h, w = h // 2, w // 2
-                skips.append((x, boc[i]))
+                skips.append(x)
+            if cfg.temporal_modules:
+                x = self._temporal_module(f"down_temporal_blocks.{i}", x, temb_all, B, Fr, h, w)
+            if i == 0:
+                tap("down0", x, boc[0], h, w)
         x = self._resnet("mid_block.resnets.0", x, None, temb_all, B, Fr, h, w)
         x = self._transformer("mid_block.attentions.0", x, kv_all, B, Fr, h, w, text_len)
         x = self._resnet("mid_block.resnets.1", x, None, temb_all, B, Fr, h, w)
+        if cfg.temporal_modules:
+            x = self._temporal_module("mid_temporal_block", x, temb_all, B, Fr, h, w)
         tap("mid", x, boc[-1], h, w)
         for i, kind in enumerate(cfg.up_block_types):
             for j in range(cfg.layers_per_block + 1):
-                skip, _ = skips.pop()
+                skip = skips.pop()
                 x = self._resnet(f"up_blocks.{i}.resnets.{j}", x, skip, temb_all, B, Fr, h, w)
                 if kind == "CrossAttnUpBlock3D":
                     x = self._transformer(f"up_blocks.{i}.attentions.{j}", x, kv_all, B, Fr, h, w, text_len)
             if i != len(boc) - 1:
                 x = self._upsample(f"up_blocks.{i}.upsamplers.0", x, B * Fr, h, w)
                 h, w = 2 * h, 2 * w
+            if cfg.temporal_modules:
+                x = self._temporal_module(f"up_temporal_blocks.{i}", x, temb_all, B, Fr, h, w)
         tap("up_out", x, boc[0], h, w)
         ss = self._gn5_scale_shift(x, None, B, Fr * h * w, P["norm_out"][0], P["norm_out"][1], cfg.norm_eps)
         if "conv_out_tc" in P:
@@ -652,6 +696,21 @@ class UNet3DConditionModel(nn.Module):
             raise ValueError(f"sample needs {self.cfg.in_channels} channels and H, W multiples of {1 << n_down}")
         if encoder_hidden_states.shape[0] != B or encoder_hidden_states.shape[-1] != self.cfg.cross_attention_dim:
             raise ValueError(f"encoder_hidden_states must be [B, L, {self.cfg.cross_attention_dim}]")
+        dev = self.device
+        out_dtype = sample.dtype
+        if self.cfg.center_input_sample:
+            sample = 2 * sample - 1.0
+        x = sample.to(device=dev, dtype=F32, non_blocking=True).contiguous()
+        if float(input_scale) == 1.0:
+            if self._scale_one is None or self._scale_one.device != dev:
+                self._scale_one = torch.ones(1, dtype=F32, device=dev)
+            scale = self._scale_one
+        else:
+            scale = torch.full((1,), float(input_scale), dtype=F32, device=dev)
+        return self._forward(x, out_dtype, timestep, encoder_hidden_states, return_dict, taps, scale=scale)
+
+    def _forward(self, x, out_dtype, timestep, encoder_hidden_states, return_dict, taps, scale=None, labels=None):
+        """What follows the argument checks in every denoiser's forward: x is the fp32 model input on the device."""
         fp = self._weights_fingerprint()
         if self._packed is not None and fp != self._param_versions:
             self._invalidate()                  # a parameter was edited in place or replaced since the last packing
@@ -659,28 +718,20 @@ class UNet3DConditionModel(nn.Module):
             self._pack()
             self._param_versions = fp
         dev = self.device
-        out_dtype = sample.dtype
+        B = x.shape[0]
         # timestep normalisation of unet.py:413-426
         if not torch.is_tensor(timestep):
             t = torch.full((B,), float(timestep), dtype=F32, device=dev)
         else:
             t = timestep.to(device=dev, dtype=F32).reshape(-1).expand(B).contiguous()
-        if self.cfg.center_input_sample:
-            sample = 2 * sample - 1.0
-        x = sample.to(device=dev, dtype=F32, non_blocking=True).contiguous()
         txt = encoder_hidden_states.to(device=dev, dtype=F32 if self.check_mode else BF16, non_blocking=True).reshape(
             -1, self.cfg.cross_attention_dim).contiguous()
-
-        if float(input_scale) == 1.0:
-            if self._scale_one is None or self._scale_one.device != dev:
-                self._scale_one = torch.ones(1, dtype=F32, device=dev)
-            scale = self._scale_one
+        vsr = self.cfg.variant == "vsr"
+        if self.use_cuda_graph and taps is None and not (vsr and self._shard is not None):   # sharded VSR: eager steps
+            # the VSR step keeps its text K/V GEMM inside the graph; the others project each prompt once (text_src)
+            out = self._graph_step(x, t, txt, scale, labels, None if vsr else encoder_hidden_states)
         else:
-            scale = torch.full((1,), float(input_scale), dtype=F32, device=dev)
-        if self.use_cuda_graph and taps is None:
-            out = self._graph_step(x, t, txt, scale, encoder_hidden_states)
-        else:
-            out = self._step(x, t, txt, taps, scale)
+            out = self._step(x, t, txt, taps, scale, labels=labels)
         out = out.to(out_dtype) if out_dtype != F32 else out.clone()   # never hand out the graph's static buffer
         if not return_dict:
             return (out,)
@@ -700,47 +751,60 @@ class UNet3DConditionModel(nn.Module):
         n = len(x) // 2
         half = x[:n]
         combined = torch.cat([half, half], dim=0)
-        out = self.forward(combined, t, encoder_hidden_states, class_labels).sample
+        return self._guided(self.forward(combined, t, encoder_hidden_states, class_labels).sample, cfg_scale)
+
+    def _guided(self, out, cfg_scale):
+        """uncond + s (cond - uncond) from the prediction of a [cond | uncond] batch (the CFG arithmetic of both
+        forward_with_cfg); channels past out_channels pass through."""
+        n = len(out) // 2
         co = self.cfg.out_channels
         eps = out[:, :co].float().contiguous()
         g = ops.cfg_combine(eps[:n], eps[n:], cfg_scale).to(out.dtype)
         return g if out.shape[1] == co else torch.cat([g, out[:, co:]], dim=1)
 
-    def _graph_step(self, x, t, txt, scale, text_src=None):
+    def _graph_step(self, x, t, txt, scale, labels, text_src):
+        """Replay of the step graph captured for this input geometry.  With ``text_src`` (the caller's prompt tensor)
+        the text K/V projections run outside the graph; without it they are part of the captured step."""
         key = (tuple(x.shape), tuple(txt.shape))
         g = self._graphs.get(key)
         if g is None:
-            g = {"x": x.clone(), "t": t.clone(), "txt": txt.clone(), "scale": scale.clone()}
+            g = {"x": x.clone(), "t": t.clone(), "txt": txt.clone(), "kv": None,
+                 "scale": None if scale is None else scale.clone(), "labels": None if labels is None else labels.clone()}
             side = torch.cuda.Stream()
             side.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(side):          # warm-up run: sets kernel attributes, fills table caches
-                g["kv"] = ops.gemm(g["txt"], self._packed["kv_w"])
-                self._step(g["x"], g["t"], g["txt"], None, g["scale"], kv_all=g["kv"])
+            with torch.cuda.stream(side):          # warm-up run: kernel attributes, table caches, zeroed VSR pad buffers
+                if text_src is not None:
+                    g["kv"] = ops.gemm(g["txt"], self._packed["kv_w"])
+                self._step(g["x"], g["t"], g["txt"], None, g["scale"], g["kv"], g["labels"])
             torch.cuda.current_stream().wait_stream(side)
             torch.cuda.synchronize()
             graph = torch.cuda.CUDAGraph()
             before = ops.LAUNCHES
             # with frame sharding the NCCL collectives of the step are captured too (same sequence on every rank)
             with torch.cuda.graph(graph):
-                g["out"] = self._step(g["x"], g["t"], g["txt"], None, g["scale"], kv_all=g["kv"])
+                g["out"] = self._step(g["x"], g["t"], g["txt"], None, g["scale"], g["kv"], g["labels"])
             g["launches"] = ops.LAUNCHES - before      # kernel nodes of ours in the captured step
             g["graph"] = graph
             self._graphs[key] = g
         g["x"].copy_(x, non_blocking=True)
         g["t"].copy_(t, non_blocking=True)
-        g["scale"].copy_(scale, non_blocking=True)
-        # text K/V projections: once per prompt tensor, outside the captured step.  A caller that passes the SAME tensor
-        # object, unmodified (version counter), step after step -- every pipeline of the reference does -- pays for the
-        # projection GEMM only on the first step.
-        seen = self._text_seen
-        hit = (text_src is not None and seen is not None and seen[0] is text_src and seen[1] == text_src._version
-               and seen[2] == key)
+        if scale is not None:
+            g["scale"].copy_(scale, non_blocking=True)
+        if labels is not None:
+            g["labels"].copy_(labels, non_blocking=True)
         extra = 0
-        if not hit:
+        if text_src is None:
             g["txt"].copy_(txt, non_blocking=True)
-            ops.gemm(g["txt"], self._packed["kv_w"], out=g["kv"])
-            extra = 1
-            self._text_seen = (text_src, text_src._version, key) if text_src is not None else None
+        else:
+            # text K/V projections: once per prompt tensor, outside the captured step.  A caller that passes the SAME
+            # tensor object, unmodified (version counter), step after step -- every pipeline of the reference does --
+            # pays for the projection GEMM only on the first step.
+            seen = self._text_seen
+            if not (seen is not None and seen[0] is text_src and seen[1] == text_src._version and seen[2] == key):
+                g["txt"].copy_(txt, non_blocking=True)
+                ops.gemm(g["txt"], self._packed["kv_w"], out=g["kv"])
+                extra = 1
+                self._text_seen = (text_src, text_src._version, key)
         self._last_graph_launches = g["launches"] + extra
         g["graph"].replay()
         return g["out"]

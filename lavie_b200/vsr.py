@@ -2,16 +2,18 @@
 super-resolution denoiser (SURVEY.md 8f row N2, BASELINE config 5).
 
 Same call signature ``forward(sample, timestep, low_res, encoder_hidden_states, class_labels) -> .sample`` and the same
-1158-key ``state_dict`` as the reference built from ``vsr/configs/unet_3d_config.json``.  It reuses every kernel of the
-base denoiser (lavie_b200/unet.py) and adds what the VSR UNet has on top:
+1158-key ``state_dict`` as the reference built from ``vsr/configs/unet_3d_config.json``.  The weight packer, the
+transformer block, the step walk, the forward body and the step graph are those of the base denoiser
+(``UNet3DConditionModel`` in lavie_b200/unet.py), which follow the config's ``variant``, ``only_cross_attention``,
+``num_class_embeds`` and ``temporal_modules`` there: the noise-level class embedding (``lavie_embedding_add``),
+transformer blocks whose first attention reads the text on the three high-resolution levels (their K/V projections join
+the one text GEMM of the step), Linear proj_in / proj_out.  This module adds what only the VSR UNet has:
 
 * ``ResnetBlock3DCNN`` -- (k,1,1) convolutions over FRAMES -- as an implicit GEMM with K = k*C on a frame-padded map
   (``lavie_frame_conv_bf16``: the same TMA box shifted by whole frames; the GroupNorm-apply + SiLU pass writes straight
-  into the padded buffer, whose pad frames stay zero);
-* the noise-level class embedding (``lavie_embedding_add``);
-* transformer blocks whose first attention reads the text on the three high-resolution levels (their K/V projections
-  join the one text GEMM of the step), Linear proj_in / proj_out, a temporal ResNet in front of every transformer;
-* a ``TemporalModule3D`` (frame ResNet (5,1,1) -> spatial ResNet -> 1x1 shift conv -> + input) behind every block.
+  into the padded buffer, whose pad frames stay zero), also the temporal ResNet in front of every transformer;
+* a ``TemporalModule3D`` (frame ResNet (5,1,1) -> spatial ResNet -> 1x1 shift conv -> + input) behind every block;
+* the forward signature with ``low_res`` and ``class_labels``, and frame sharding over the NCCL back end only.
 
 There is no PyTorch compute fallback; the module raises on non-CUDA parameters like the base one.
 """
@@ -22,9 +24,8 @@ from typing import Dict, Optional, Union
 import torch
 
 from . import ops
-from .config import VSR_CONFIG, UNetConfig, param_spec
-from .packing import head_pitch, interleave_geglu, pack_conv1x1, pack_conv3x3, pack_upsample_conv3x3, pad_heads
-from .unet import BF16, F32, UNet3DConditionModel, UNet3DConditionOutput
+from .config import VSR_CONFIG, UNetConfig
+from .unet import BF16, F32, UNet3DConditionModel
 
 
 def pack_frame_conv(w: torch.Tensor) -> torch.Tensor:
@@ -36,11 +37,11 @@ def pack_frame_conv(w: torch.Tensor) -> torch.Tensor:
 class UNet3DVSRModel(UNet3DConditionModel):
     """B200-native LaVie VSR denoiser (bf16 activations, fp32 accumulation)."""
     _VARIANTS = ("vsr",)
+    _TAPS = ("down0", "mid")            # behind the first and the mid TemporalModule3D (tests/golden/make_golden_vsr.py)
 
     def __init__(self, config: UNetConfig = VSR_CONFIG, use_cuda_graph: bool = True):
         super().__init__(config, use_cuda_graph=use_cuda_graph, check_mode=False)
         self._padbufs: Dict[tuple, torch.Tensor] = {}
-        self._graph_ok = True
 
     def set_frame_sharding(self, group=None, backend: str = "nccl", frame_counts=None):
         """Frame sharding of the VSR denoiser (BASELINE config 5): every rank of `group` holds F / P consecutive frames of
@@ -51,137 +52,11 @@ class UNet3DVSRModel(UNet3DConditionModel):
         if group is not None and (backend != "nccl" or frame_counts is not None):
             raise NotImplementedError("the VSR denoiser shards equal frame counts over the NCCL back end only")
         super().set_frame_sharding(group, backend="nccl" if group is not None else "p2p")
-        self._graph_ok = self._shard is None
         self._padbufs = {}          # pad frames that held halos must not be mistaken for the zero padding of an un-sharded run
 
     def _invalidate(self):
         super()._invalidate()
         self._padbufs = {}
-
-    # ------------------------------------------------------------------ weight packing
-    def _pack(self):
-        sd = {k: v.detach() for k, v in self.state_dict().items()}
-        spec = param_spec(self.cfg)
-        missing = [k for k in spec if k not in sd]
-        if missing:
-            raise RuntimeError(f"state_dict no longer has the reference layout (first missing key: {missing[0]})")
-        dev = self.device
-        if dev.type != "cuda":
-            raise RuntimeError("lavie_b200.UNet3DVSRModel runs on CUDA (sm_100a) only; move it with .to('cuda')")
-        heads = self.cfg.heads
-        P: Dict[str, object] = {}
-
-        def f32(k):
-            return sd[k].to(device=dev, dtype=F32).contiguous()
-
-        def b16(t):
-            return t.to(device=dev, dtype=BF16).contiguous()
-
-        temb_w, temb_b, temb_slices = [], [], {}
-        kv_w = []
-        state = {"temb": 0, "kv": 0}
-
-        def add_temb(p, cout):
-            temb_w.append(sd[f"{p}.time_emb_proj.weight"])
-            temb_b.append(sd[f"{p}.time_emb_proj.bias"])
-            temb_slices[p] = (state["temb"], cout)
-            state["temb"] += cout
-
-        def add_kv(b, a, hp):
-            kv_w.append(pad_heads(sd[f"{b}.{a}.to_k.weight"], heads))
-            kv_w.append(pad_heads(sd[f"{b}.{a}.to_v.weight"], heads))
-            off = state["kv"]
-            state["kv"] += 2 * hp
-            return off
-
-        for key, shape in spec.items():
-            if not key.endswith(".conv1.weight"):
-                continue
-            p = key[: -len(".conv1.weight")]
-            r = {"g1": f32(f"{p}.norm1.weight"), "b1": f32(f"{p}.norm1.bias"), "cb1": f32(f"{p}.conv1.bias"),
-                 "g2": f32(f"{p}.norm2.weight"), "b2": f32(f"{p}.norm2.bias"), "cb2": f32(f"{p}.conv2.bias")}
-            if len(shape) == 5:                                   # ResnetBlock3DCNN (vsr/models/resnet.py:220-316)
-                r["k"] = shape[2]
-                r["w1"] = b16(pack_frame_conv(sd[f"{p}.conv1.weight"]))
-                r["w2"] = b16(pack_frame_conv(sd[f"{p}.conv2.weight"]))
-            else:                                                 # ResnetBlock3D
-                r["w1"] = b16(pack_conv3x3(sd[f"{p}.conv1.weight"], dtype=None))
-                r["w2"] = b16(pack_conv3x3(sd[f"{p}.conv2.weight"], dtype=None))
-                if f"{p}.conv_shortcut.weight" in sd:
-                    r["wsc"] = b16(pack_conv1x1(sd[f"{p}.conv_shortcut.weight"], dtype=None))
-                    r["bsc"] = f32(f"{p}.conv_shortcut.bias")
-                if "temporal_block" in p:                         # TemporalModule3D builds it with the default eps
-                    r["eps"] = 1e-6
-            if f"{p}.time_emb_proj.weight" in sd:
-                add_temb(p, shape[0])
-            P[p] = r
-
-        for key in spec:
-            if not key.endswith(".proj_in.weight"):
-                continue
-            p = key[: -len(".proj_in.weight")]
-            b = f"{p}.transformer_blocks.0"
-            C = sd[f"{p}.norm.weight"].shape[0]
-            d = C // heads
-            hp = heads * head_pitch(d)
-            only_cross = sd[f"{b}.attn1.to_k.weight"].shape[1] != C or (
-                self.cfg.cross_attention_dim == C and self._only_cross_for(p))
-            t = {"C": C, "d": d, "pitch": head_pitch(d), "hp": hp, "only_cross": only_cross,
-                 "gn_g": f32(f"{p}.norm.weight"), "gn_b": f32(f"{p}.norm.bias"),
-                 "w_in": b16(sd[f"{p}.proj_in.weight"]), "b_in": f32(f"{p}.proj_in.bias"),
-                 "w_out": b16(sd[f"{p}.proj_out.weight"]), "b_out": f32(f"{p}.proj_out.bias")}
-            for n in ("norm1", "norm2", "norm_temporal", "norm3"):
-                t[f"{n}_g"] = f32(f"{b}.{n}.weight")
-                t[f"{n}_b"] = f32(f"{b}.{n}.bias")
-            if only_cross:
-                t["attn1_q"] = b16(pad_heads(sd[f"{b}.attn1.to_q.weight"], heads))
-                t["attn1_kv_off"] = add_kv(b, "attn1", hp)
-            else:
-                t["attn1_qkv"] = b16(torch.cat([pad_heads(sd[f"{b}.attn1.to_{x}.weight"], heads) for x in "qkv"], 0))
-            t["attn_temporal_qkv"] = b16(torch.cat([pad_heads(sd[f"{b}.attn_temporal.to_{x}.weight"], heads)
-                                                    for x in "qkv"], 0))
-            for a in ("attn1", "attn2", "attn_temporal"):
-                t[f"{a}_wo"] = b16(sd[f"{b}.{a}.to_out.0.weight"])
-                t[f"{a}_bo"] = f32(f"{b}.{a}.to_out.0.bias")
-            t["attn2_q"] = b16(pad_heads(sd[f"{b}.attn2.to_q.weight"], heads))
-            t["kv_off"] = add_kv(b, "attn2", hp)
-            wi, bi = interleave_geglu(sd[f"{b}.ff.net.0.proj.weight"], sd[f"{b}.ff.net.0.proj.bias"])
-            t["ff1_w"], t["ff1_b"] = b16(wi), bi.to(device=dev, dtype=F32).contiguous()
-            t["ff2_w"], t["ff2_b"] = b16(sd[f"{b}.ff.net.2.weight"]), f32(f"{b}.ff.net.2.bias")
-            t["rel_emb"] = f32(f"{b}.attn_temporal.time_rel_pos_bias.relative_attention_bias.weight")
-            t["freqs"] = f32(f"{b}.attn_temporal.rotary_emb.freqs")
-            P[p] = t
-
-        for key in spec:
-            if key.endswith(".shift_conv.weight"):
-                p = key[: -len(".shift_conv.weight")]
-                P[f"{p}.shift_conv"] = (b16(pack_conv1x1(sd[key], dtype=None)), f32(f"{p}.shift_conv.bias"))
-        n_levels = len(self.cfg.block_out_channels)
-        for i in range(n_levels - 1):
-            for side, name in (("down_blocks", "downsamplers"), ("up_blocks", "upsamplers")):
-                q = f"{side}.{i}.{name}.0.conv"
-                P[q] = (b16(pack_conv3x3(sd[f"{q}.weight"], dtype=None)), f32(f"{q}.bias"))
-                if name == "upsamplers":
-                    P[f"{q}4"] = pack_upsample_conv3x3(sd[f"{q}.weight"]).to(dev)
-        boc0 = self.cfg.block_out_channels[0]
-        P["conv_in"] = (f32("conv_in.weight"), f32("conv_in.bias"))
-        P["conv_in_tc"] = (ops.pack_conv_in(sd["conv_in.weight"], dev), f32("conv_in.bias"))
-        co = sd["conv_out.weight"].shape[0]
-        wp = torch.zeros((ops.CONV_OUT_PAD, 9 * boc0), dtype=F32)
-        wp[:co] = pack_conv3x3(sd["conv_out.weight"].float().cpu(), dtype=None)
-        bp = torch.zeros(ops.CONV_OUT_PAD, dtype=F32)
-        bp[:co] = sd["conv_out.bias"].float().cpu()
-        P["conv_out_tc"] = (wp.to(device=dev, dtype=BF16).contiguous(), bp.to(dev), co)
-        P["norm_out"] = (f32("conv_norm_out.weight"), f32("conv_norm_out.bias"))
-        P["time1"] = (b16(sd["time_embedding.linear_1.weight"]), f32("time_embedding.linear_1.bias"))
-        P["time2"] = (b16(sd["time_embedding.linear_2.weight"]), f32("time_embedding.linear_2.bias"))
-        P["class_emb"] = f32("class_embedding.weight")
-        P["temb_w"] = b16(torch.cat(temb_w, 0))
-        P["temb_b"] = torch.cat(temb_b, 0).to(device=dev, dtype=F32).contiguous()
-        P["temb_slices"] = temb_slices
-        P["kv_w"] = b16(torch.cat(kv_w, 0))
-        self._packed = P
-        return P
 
     def _only_cross_for(self, p: str) -> bool:
         """only_cross_attention of the level a transformer prefix belongs to (vsr/models/unet.py:134-139, 272)."""
@@ -251,115 +126,6 @@ class UNet3DVSRModel(UNet3DConditionModel):
         w, b = self._packed[f"{p}.shift_conv"]
         return ops.gemm(h, w, bias=b, residual=x, stats=True)
 
-    def _transformer_vsr(self, p, x, kv_all, B, Fr, H, W, text_len):
-        """Transformer3DModel.forward + BasicTransformerBlock.forward of the VSR tree (vsr/models/attention.py:386-438,
-        556-593)."""
-        t = self._packed[p]
-        heads, d, pitch, hp = self.cfg.heads, t["d"], t["pitch"], t["hp"]
-        NF, HW = B * Fr, H * W
-        x = self._resnet_cnn(f"{p}.resblock_temporal", x, None, B, Fr, HW)
-        h = ops.groupnorm(x, NF, HW, t["gn_g"], t["gn_b"], 1e-6, silu=False)           # per-frame GN (4-D input)
-        tok = ops.gemm(h, t["w_in"], bias=t["b_in"])
-        n = ops.layernorm(tok, t["norm1_g"], t["norm1_b"])
-        if t["only_cross"]:                                    # attn1 reads the text (only_cross_attention levels)
-            q = ops.gemm(n, t["attn1_q"])
-            ko = t["attn1_kv_off"]
-            a = ops.attention(q, kv_all[:, ko:ko + hp], kv_all[:, ko + hp:ko + 2 * hp], NF, heads, HW, text_len, d, pitch,
-                              kv_batch_div=Fr)
-        else:
-            qkv = ops.gemm(n, t["attn1_qkv"])
-            a = ops.attention(qkv[:, :hp], qkv[:, hp:2 * hp], qkv[:, 2 * hp:], NF, heads, HW, HW, d, pitch)
-        tok = ops.gemm(a, t["attn1_wo"], bias=t["attn1_bo"], residual=tok)
-        n = ops.layernorm(tok, t["norm2_g"], t["norm2_b"])
-        q = ops.gemm(n, t["attn2_q"])
-        ko = t["kv_off"]
-        a = ops.attention(q, kv_all[:, ko:ko + hp], kv_all[:, ko + hp:ko + 2 * hp], NF, heads, HW, text_len, d, pitch,
-                          kv_batch_div=Fr)
-        tok = ops.gemm(a, t["attn2_wo"], bias=t["attn2_bo"], residual=tok)
-        if self._shard is None:
-            n = ops.layernorm(tok, t["norm_temporal_g"], t["norm_temporal_b"])
-            qkv = ops.gemm(n, t["attn_temporal_qkv"])
-            rope, bias = self._frame_tables(p, Fr)
-            a = ops.temporal_attention(qkv, B, Fr, HW, heads, d, pitch, rope, bias)
-            tok = ops.gemm(a, t["attn_temporal_wo"], bias=t["attn_temporal_bo"], residual=tok)
-        else:
-            # frame-sharded: all-to-all to pixel sharding (every rank gets ALL frames of HW/P pixels), attend, and back
-            import torch.distributed as dist
-            group, P, _ = self._shard
-            assert B == 1 and HW % P == 0, "frame sharding runs one CFG half per rank and needs H*W divisible by P"
-            hwp = HW // P
-            send = ops.layernorm_scatter(tok, t["norm_temporal_g"], t["norm_temporal_b"], HW, hwp)   # [P, F_loc, hwp, C]
-            recv = torch.empty_like(send)                                                             # [F, hwp, C]
-            dist.all_to_all_single(recv, send, group=group)
-            qkv = ops.gemm(recv, t["attn_temporal_qkv"])
-            rope, bias = self._frame_tables(p, Fr * P)
-            a = ops.temporal_attention(qkv, 1, Fr * P, hwp, heads, d, pitch, rope, bias)
-            y = ops.gemm(a, t["attn_temporal_wo"], bias=t["attn_temporal_bo"])                        # [F, hwp, C]
-            back = torch.empty_like(y)                                                                # [P, F_loc, hwp, C]
-            dist.all_to_all_single(back, y, group=group)
-            tok = ops.add_gathered(tok, back, HW, hwp)
-        n = ops.layernorm(tok, t["norm3_g"], t["norm3_b"])
-        g = ops.gemm(n, t["ff1_w"], bias=t["ff1_b"], geglu=True)
-        tok = ops.gemm(g, t["ff2_w"], bias=t["ff2_b"], residual=tok)
-        return ops.gemm(tok, t["w_out"], bias=t["b_out"], residual=x, stats=True)
-
-    def _step_vsr(self, sample7: torch.Tensor, t: torch.Tensor, text: torch.Tensor, labels: torch.Tensor,
-                  taps: Optional[dict] = None):
-        """sample7 fp32 [B,7,F,H,W] (latent | low-res frames), t fp32 [B], text bf16 [B*L, 1024], labels int64 [B]."""
-        P = self._packed
-        cfg = self.cfg
-        B, _, Fr, H, W = sample7.shape
-        text_len = text.shape[0] // B
-        boc = cfg.block_out_channels
-        n_levels = len(boc)
-
-        def tap(name, x, C, h, w):
-            if taps is not None:
-                taps[name] = x.float().reshape(B, Fr, h, w, C).permute(0, 4, 1, 2, 3).contiguous()
-
-        temb = ops.timestep_embedding(t, boc[0])
-        h1 = ops.linear_smallm(temb, P["time1"][0], P["time1"][1], silu_out=True)
-        emb = ops.linear_smallm(h1, P["time2"][0], P["time2"][1])
-        ops.embedding_add(emb, P["class_emb"], labels)
-        temb_all = ops.linear_smallm(emb, P["temb_w"], P["temb_b"], silu_in=True)
-        kv_all = ops.gemm(text, P["kv_w"])
-
-        x = ops.conv_in_tc(sample7, P["conv_in_tc"][0], P["conv_in_tc"][1], None)
-        skips = [x]
-        h, w = H, W
-        for i, kind in enumerate(cfg.down_block_types):
-            for j in range(cfg.layers_per_block):
-                x = self._resnet(f"down_blocks.{i}.resnets.{j}", x, None, temb_all, B, Fr, h, w)
-                if kind == "CrossAttnDownBlock3D":
-                    x = self._transformer_vsr(f"down_blocks.{i}.attentions.{j}", x, kv_all, B, Fr, h, w, text_len)
-                skips.append(x)
-            if i != n_levels - 1:
-                wd, bd = P[f"down_blocks.{i}.downsamplers.0.conv"]
-                x = ops.conv3x3(x, B * Fr, h, w, wd, stride=2, bias=bd, stats=True)
-                h, w = h // 2, w // 2
-                skips.append(x)
-            x = self._temporal_module(f"down_temporal_blocks.{i}", x, temb_all, B, Fr, h, w)
-            if i == 0:
-                tap("down0", x, boc[0], h, w)
-        x = self._resnet("mid_block.resnets.0", x, None, temb_all, B, Fr, h, w)
-        x = self._transformer_vsr("mid_block.attentions.0", x, kv_all, B, Fr, h, w, text_len)
-        x = self._resnet("mid_block.resnets.1", x, None, temb_all, B, Fr, h, w)
-        x = self._temporal_module("mid_temporal_block", x, temb_all, B, Fr, h, w)
-        tap("mid", x, boc[-1], h, w)
-        for i, kind in enumerate(cfg.up_block_types):
-            for j in range(cfg.layers_per_block + 1):
-                skip = skips.pop()
-                x = self._resnet(f"up_blocks.{i}.resnets.{j}", x, skip, temb_all, B, Fr, h, w)
-                if kind == "CrossAttnUpBlock3D":
-                    x = self._transformer_vsr(f"up_blocks.{i}.attentions.{j}", x, kv_all, B, Fr, h, w, text_len)
-            if i != n_levels - 1:
-                x = self._upsample(f"up_blocks.{i}.upsamplers.0", x, B * Fr, h, w)
-                h, w = 2 * h, 2 * w
-            x = self._temporal_module(f"up_temporal_blocks.{i}", x, temb_all, B, Fr, h, w)
-        ss = self._gn5_scale_shift(x, None, B, Fr * h * w, P["norm_out"][0], P["norm_out"][1], cfg.norm_eps)
-        wp, bp, co = P["conv_out_tc"]
-        return ops.conv_out_tc(x, ss, B, Fr, h, w, wp, bp, co)
-
     # ------------------------------------------------------------------ public forward
     @torch.no_grad()
     def forward(self, sample: torch.Tensor, timestep: Union[torch.Tensor, float, int], low_res: torch.Tensor,
@@ -388,30 +154,10 @@ class UNet3DVSRModel(UNet3DConditionModel):
         if bool((labels > self.cfg.max_noise_level).any()):
             raise ValueError(f"`noise_level` has to be <= {self.cfg.max_noise_level} but is {class_labels}")   # :499
         labels = labels.expand(B).contiguous().to(dev, non_blocking=True)
-        fp = self._weights_fingerprint()
-        if self._packed is not None and fp != self._param_versions:
-            self._invalidate()
-        if self._packed is None:
-            self._pack()
-            self._param_versions = fp
-        out_dtype = sample.dtype
-        if not torch.is_tensor(timestep):
-            t = torch.full((B,), float(timestep), dtype=F32, device=dev)
-        else:
-            t = timestep.to(device=dev, dtype=F32).reshape(-1).expand(B).contiguous()
         x = torch.cat([sample.to(device=dev, dtype=F32), low_res.to(device=dev, dtype=F32)], dim=1)     # unet.py:446
         if self.cfg.center_input_sample:
             x = 2 * x - 1.0
-        txt = encoder_hidden_states.to(device=dev, dtype=BF16, non_blocking=True).reshape(
-            -1, self.cfg.cross_attention_dim).contiguous()
-        if self.use_cuda_graph and self._graph_ok and taps is None:
-            out = self._graph_step_vsr(x, t, txt, labels)
-        else:
-            out = self._step_vsr(x, t, txt, labels, taps)
-        out = out.to(out_dtype) if out_dtype != F32 else out.clone()
-        if not return_dict:
-            return (out,)
-        return UNet3DConditionOutput(sample=out)
+        return self._forward(x, sample.dtype, timestep, encoder_hidden_states, return_dict, taps, labels=labels)
 
     @torch.no_grad()
     def forward_with_cfg(self, x, t, low_res, encoder_hidden_states=None, class_labels=20, cfg_scale: float = 4.0,
@@ -420,33 +166,4 @@ class UNet3DVSRModel(UNet3DConditionModel):
         noise is returned for both halves."""
         n = len(x) // 2
         combined = torch.cat([x[:n], x[:n]], dim=0)
-        out = self.forward(combined, t, low_res, encoder_hidden_states, class_labels).sample
-        eps = out[:, :4].float().contiguous()
-        g = ops.cfg_combine(eps[:n], eps[n:], cfg_scale).to(out.dtype)
-        return g if out.shape[1] == 4 else torch.cat([g, out[:, 4:]], dim=1)
-
-    def _graph_step_vsr(self, x, t, txt, labels):
-        key = (tuple(x.shape), tuple(txt.shape))
-        g = self._graphs.get(key)
-        if g is None:
-            g = {"x": x.clone(), "t": t.clone(), "txt": txt.clone(), "labels": labels.clone()}
-            side = torch.cuda.Stream()
-            side.wait_stream(torch.cuda.current_stream())
-            with torch.cuda.stream(side):          # warm-up run: kernel attributes, table caches, zeroed pad buffers
-                self._step_vsr(g["x"], g["t"], g["txt"], g["labels"])
-            torch.cuda.current_stream().wait_stream(side)
-            torch.cuda.synchronize()
-            graph = torch.cuda.CUDAGraph()
-            before = ops.LAUNCHES
-            with torch.cuda.graph(graph):
-                g["out"] = self._step_vsr(g["x"], g["t"], g["txt"], g["labels"])
-            g["launches"] = ops.LAUNCHES - before
-            g["graph"] = graph
-            self._graphs[key] = g
-        self._last_graph_launches = g["launches"]
-        g["x"].copy_(x, non_blocking=True)
-        g["t"].copy_(t, non_blocking=True)
-        g["txt"].copy_(txt, non_blocking=True)
-        g["labels"].copy_(labels, non_blocking=True)
-        g["graph"].replay()
-        return g["out"]
+        return self._guided(self.forward(combined, t, low_res, encoder_hidden_states, class_labels).sample, cfg_scale)
