@@ -346,6 +346,13 @@ int lavie_activation_bf16(void* x, long long n, int kind, lavie_stream_t stream)
  * probabilities of the VAE decoder's single-head mid-block attention (diffusers AttentionBlock), whose Q K^T and P V
  * products are plain GEMMs. */
 int lavie_softmax_rows_bf16(void* s, int ld, long long rows, int n, float scale, lavie_stream_t stream);
+/* One-head attention with d = 512, per frame: o = softmax(q k^T) v, the single-head mid-block attention of the
+ * x4-upscaler VAE decoder (diffusers AttentionBlock, 512 channels) at any token count S >= 1.  q, k, v, o are bf16
+ * row-major [frames * S, 512] views with row strides ld* (multiples of 8, >= 512) and 16-byte aligned bases; frame f
+ * occupies rows [f * S, (f + 1) * S).  The 512^-1/2 scale must already be folded into q.  fp32 accumulation,
+ * deterministic, writes only the 512 columns of each o row.  frames <= 65535. */
+int lavie_attention_wide_bf16(const void* q, int ldq, const void* k, int ldk, const void* v, int ldv, void* o, int ldo,
+                              int frames, int S, lavie_stream_t stream);
 /* AutoencoderKL.post_quant_conv (1x1, 4 -> 4; mirror vsr/models/autoencoder_kl.py:183) on an fp32 [N, Cin, pixels] map,
  * with decode_latents' 1/0.18215 folded in: out[n, co, p] = bias[co] + sum_ci w[co, ci] * scale * x[n, ci, p]. */
 int lavie_pointwise_conv_nchw_f32(const float* x, const float* w, const float* bias, float scale, int N, int Cin, int Cout,

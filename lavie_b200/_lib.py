@@ -91,6 +91,7 @@ SIGNATURES = {
     "lavie_causal_attention_small": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_float, _P, c_int, _P]),
     "lavie_activation_bf16": (c_int, [_P, c_longlong, c_int, _P]),
     "lavie_softmax_rows_bf16": (c_int, [_P, c_int, c_longlong, c_int, c_float, _P]),
+    "lavie_attention_wide_bf16": (c_int, [_P, c_int, _P, c_int, _P, c_int, _P, c_int, c_int, c_int, _P]),
     "lavie_image_to_uint8": (c_int, [_P, c_int, c_longlong, _P, _P]),
     "lavie_pointwise_conv_nchw_f32": (c_int, [_P, _P, _P, c_float, c_int, c_int, c_int, c_longlong, _P, _P]),
     "lavie_groupnorm_finalize_colsums_seg": (c_int, [_P, c_int, c_int, _P, c_int, c_int, c_int, c_int, c_int, _P, _P,

@@ -7,7 +7,14 @@ vsr/models/autoencoder_kl.py:179-192).  This module keeps the decode-side ``stat
 runs the published Stable-Diffusion VAE decoder as C-ABI launches that reuse the denoiser's kernels: implicit-GEMM 3x3
 convs on tcgen05, per-frame GroupNorm + SiLU, nearest-x2 upsample; the single-head 2560-token mid-block attention is two
 GEMMs around a row-softmax kernel (Q K^T per frame, P V against V^T produced directly by a GEMM).  bf16 activations, fp32
-accumulation.  No CPU fallback."""
+accumulation.  No CPU fallback.
+
+The same class runs the x4-upscaler VAE that the VSR pipeline decodes with (``VAEDecoder.x4_upscaler()``, published
+``vae/config.json`` of the x4 upscaler: block_out_channels (128, 256, 512), layers_per_block 2, 32 groups, scaling
+factor 0.08333, two upsamplers, so the output is x4).  Its mid-block attention sees h * w tokens per frame at the
+latent resolution (163 840 at 320x512), far beyond a materialised score matrix: it runs the fused single-head d = 512
+kernel of ``vae_attention`` instead.  Frames are decoded in groups sized from the geometry so that no tensor of any
+launch passes 2^31 elements."""
 from __future__ import annotations
 
 import math
@@ -21,14 +28,24 @@ from torch import nn
 from . import ops
 from .packing import pack_conv1x1, pack_conv3x3, pack_upsample_conv3x3
 from .synthetic import _gen
+from .vae_attention import attention_wide
 
 BF16 = torch.bfloat16
 F32 = torch.float32
 UP_CHANNELS = (512, 512, 256, 128)          # reversed block_out_channels of the SD VAE
 SCALING = 0.18215                            # pipeline_videogen.py:424
+SD_BLOCK_OUT = (128, 256, 512, 512)
+# stabilityai/stable-diffusion-x4-upscaler vae/config.json
+X4_BLOCK_OUT = (128, 256, 512)
+X4_SCALING = 0.08333
+MAX_LAUNCH_ELEMENTS = 2 ** 31 - 1           # largest tensor one launch may address with 32-bit element indices
 
 
-def vae_decoder_param_spec() -> "OrderedDict[str, Tuple[int, ...]]":
+def vae_decoder_param_spec(block_out_channels=SD_BLOCK_OUT, layers_per_block: int = 2
+                           ) -> "OrderedDict[str, Tuple[int, ...]]":
+    """Decode-side parameters of diffusers' AutoencoderKL (0.16 names).  Default: the Stable Diffusion VAE."""
+    up_channels = tuple(reversed(block_out_channels))
+    top = up_channels[0]
     spec: "OrderedDict[str, Tuple[int, ...]]" = OrderedDict()
 
     def conv(p, co, ci, k):
@@ -48,31 +65,33 @@ def vae_decoder_param_spec() -> "OrderedDict[str, Tuple[int, ...]]":
             conv(f"{p}.conv_shortcut", co, ci, 1)
 
     conv("post_quant_conv", 4, 4, 1)
-    conv("decoder.conv_in", 512, 4, 3)
-    resnet("decoder.mid_block.resnets.0", 512, 512)
+    conv("decoder.conv_in", top, 4, 3)
+    resnet("decoder.mid_block.resnets.0", top, top)
     a = "decoder.mid_block.attentions.0"
-    norm(f"{a}.group_norm", 512)
+    norm(f"{a}.group_norm", top)
     for n in ("query", "key", "value", "proj_attn"):
-        spec[f"{a}.{n}.weight"] = (512, 512)
-        spec[f"{a}.{n}.bias"] = (512,)
-    resnet("decoder.mid_block.resnets.1", 512, 512)
-    prev = 512
-    for i, c in enumerate(UP_CHANNELS):
-        for j in range(3):
+        spec[f"{a}.{n}.weight"] = (top, top)
+        spec[f"{a}.{n}.bias"] = (top,)
+    resnet("decoder.mid_block.resnets.1", top, top)
+    prev = top
+    for i, c in enumerate(up_channels):
+        for j in range(layers_per_block + 1):
             resnet(f"decoder.up_blocks.{i}.resnets.{j}", prev if j == 0 else c, c)
-        if i != len(UP_CHANNELS) - 1:
+        if i != len(up_channels) - 1:
             conv(f"decoder.up_blocks.{i}.upsamplers.0.conv", c, c, 3)
         prev = c
-    norm("decoder.conv_norm_out", 128)
-    conv("decoder.conv_out", 3, 128, 3)
+    norm("decoder.conv_norm_out", up_channels[-1])
+    conv("decoder.conv_out", 3, up_channels[-1], 3)
     return spec
 
 
-def vae_synthetic_state_dict(seed: int = 0):
+def vae_synthetic_state_dict(seed: int = 0, block_out_channels=SD_BLOCK_OUT):
+    """Seeded decoder weights; ``block_out_channels=X4_BLOCK_OUT`` draws the x4-upscaler layout."""
     sd = OrderedDict()
-    spec = vae_decoder_param_spec()
+    spec = vae_decoder_param_spec(block_out_channels)
+    tag = "vae:" if tuple(block_out_channels) == SD_BLOCK_OUT else f"vae{tuple(block_out_channels)}:"
     for key, shape in spec.items():
-        g = _gen(seed, "vae:" + key)
+        g = _gen(seed, tag + key)
         if ".norm" in key or "group_norm" in key or "conv_norm_out" in key:
             t = 0.1 * torch.randn(shape, generator=g) + (1.0 if key.endswith("weight") else 0.0)
         else:
@@ -102,12 +121,23 @@ def load_vae_state_dict(module: "VAEDecoder", sd, strict: bool = True):
 
 
 class VAEDecoder(nn.Module):
-    """``decode(z).sample`` of the Stable Diffusion VAE + the pipelines' ``decode_latents``."""
+    """``decode(z).sample`` of an AutoencoderKL decoder + the pipelines' ``decode_latents``.  No arguments: the Stable
+    Diffusion VAE (x8); ``VAEDecoder.x4_upscaler()``: the x4-upscaler VAE of the VSR pipeline."""
 
-    def __init__(self):
+    def __init__(self, block_out_channels=SD_BLOCK_OUT, scaling_factor: float = SCALING, layers_per_block: int = 2):
         super().__init__()
-        self.config = SimpleNamespace(scaling_factor=SCALING, latent_channels=4)
-        for key, shape in vae_decoder_param_spec().items():
+        block_out_channels = tuple(int(c) for c in block_out_channels)
+        self.config = SimpleNamespace(scaling_factor=scaling_factor, latent_channels=4,
+                                      block_out_channels=block_out_channels, layers_per_block=layers_per_block,
+                                      norm_num_groups=32)
+        self.up_channels = tuple(reversed(block_out_channels))
+        self.upscale = 2 ** (len(block_out_channels) - 1)
+        # the SD VAE keeps its GEMM + row-softmax attention (2560 tokens at its 40x64 latent); every other configuration
+        # runs the fused wide kernel, which has no token limit
+        self.wide_attention = block_out_channels != SD_BLOCK_OUT
+        if self.wide_attention and self.up_channels[0] != 512:
+            raise ValueError("the fused mid-block attention needs block_out_channels[-1] == 512")
+        for key, shape in vae_decoder_param_spec(block_out_channels, layers_per_block).items():
             prefix, leaf = key.rsplit(".", 1)
             cur = self
             for p in prefix.split("."):
@@ -119,6 +149,11 @@ class VAEDecoder(nn.Module):
             cur.register_parameter(leaf, nn.Parameter(torch.empty(shape), requires_grad=False))
         self._packed = None
         self.register_load_state_dict_post_hook(lambda module, incompatible: module._invalidate())
+
+    @classmethod
+    def x4_upscaler(cls) -> "VAEDecoder":
+        """The VAE of the x4 upscaler (the VSR pipeline's decoder): [N,4,h,w] -> [N,3,4h,4w]."""
+        return cls(X4_BLOCK_OUT, X4_SCALING)
 
     def _invalidate(self):
         self._packed = None
@@ -159,7 +194,7 @@ class VAEDecoder(nn.Module):
                 p = key[: -len(".weight")]
                 P[p] = (b16(pack_conv3x3(sd[key], dtype=None)), f32(f"{p}.bias"), pack_upsample_conv3x3(sd[key]).to(dev))
         a = "decoder.mid_block.attentions.0"
-        C = 512
+        C = self.up_channels[0]
         s = C ** -0.5                                   # folded into the query projection: scores leave the GEMM scaled
         P[a] = {"g": f32(f"{a}.group_norm.weight"), "b": f32(f"{a}.group_norm.bias"),
                 "w_q": b16(sd[f"{a}.query.weight"].float() * s),
@@ -167,9 +202,13 @@ class VAEDecoder(nn.Module):
                 "w_k": b16(sd[f"{a}.key.weight"]), "b_k": f32(f"{a}.key.bias"),
                 "w_v": b16(sd[f"{a}.value.weight"]), "b_v": f32(f"{a}.value.bias"),
                 "w_o": b16(sd[f"{a}.proj_attn.weight"]), "b_o": f32(f"{a}.proj_attn.bias")}
+        if self.wide_attention:                         # q, k, v from one GEMM: [rows, 3C], read as strided views
+            t = P[a]
+            t["w_qkv"] = torch.cat([t.pop("w_q"), t.pop("w_k"), t.pop("w_v")]).contiguous()
+            t["b_qkv"] = torch.cat([t.pop("b_q"), t.pop("b_k"), t.pop("b_v")]).contiguous()
         P["pq"] = (f32("post_quant_conv.weight").reshape(4, 4).contiguous(), f32("post_quant_conv.bias"))
         P["conv_in"] = (f32("decoder.conv_in.weight"), f32("decoder.conv_in.bias"))
-        wp = torch.zeros((ops.CONV_OUT_PAD, 9 * 128), dtype=F32)
+        wp = torch.zeros((ops.CONV_OUT_PAD, 9 * self.up_channels[-1]), dtype=F32)
         wp[:3] = pack_conv3x3(sd["decoder.conv_out.weight"].float().cpu(), dtype=None)
         bp = torch.zeros(ops.CONV_OUT_PAD, dtype=F32)
         bp[:3] = sd["decoder.conv_out.bias"].float().cpu()
@@ -192,6 +231,10 @@ class VAEDecoder(nn.Module):
         t = self._packed["decoder.mid_block.attentions.0"]
         C = 512
         n = ops.groupnorm(x, N, HW, t["g"], t["b"], 1e-6, silu=False)
+        if self.wide_attention:
+            qkv = ops.gemm(n, t["w_qkv"], bias=t["b_qkv"])                # [rows, 3C]; q already scaled by C^-1/2
+            o = attention_wide(qkv[:, :C], qkv[:, C:2 * C], qkv[:, 2 * C:], N, HW)
+            return ops.gemm(o, t["w_o"], bias=t["b_o"], residual=x, stats=True)
         if HW % 8:
             raise ValueError("the VAE mid-block attention needs h * w to be a multiple of 8")
         q = ops.gemm(n, t["w_q"], bias=t["b_q"])                          # already scaled by C^-1/2
@@ -206,27 +249,42 @@ class VAEDecoder(nn.Module):
             ops.gemm(s, vt, bias=t["b_v"], out=o[rows])
         return ops.gemm(o, t["w_o"], bias=t["b_o"], residual=x, stats=True)
 
-    @torch.no_grad()
-    def decode(self, z: torch.Tensor, return_dict: bool = True, scale: float = 1.0, as_uint8: bool = False):
-        """AutoencoderKL.decode (mirror vsr/models/autoencoder_kl.py:179-198): z [N,4,h,w] -> ``.sample`` [N,3,8h,8w] in
-        z's dtype.  ``scale`` multiplies z first (decode_latents' 1/0.18215); ``as_uint8`` returns the pipelines' uint8
-        frames [N, 8h, 8w, 3] instead."""
-        if z.dim() != 4 or z.shape[1] != 4:
-            raise ValueError(f"z must be [N,4,h,w], got {tuple(z.shape)}")
-        P = self._packed or self._pack()
-        dev = self.device
-        N, _, h, w = z.shape
-        zin = z.to(device=dev, dtype=F32).contiguous()
+    def frame_elements(self, h: int, w: int) -> int:
+        """Largest tensor, in elements per frame, that any launch of a decode at an h x w latent touches: the mid-block
+        q/k/v rows at the latent resolution, and every level's maps at the channel count they enter and leave with
+        (an upsampled map keeps the channels of the level below it)."""
+        top = self.up_channels[0]
+        most = 3 * top * h * w
+        prev, H, W = top, h, w
+        for i, c in enumerate(self.up_channels):
+            most = max(most, max(prev, c) * H * W)
+            if i != len(self.up_channels) - 1:
+                H, W = 2 * H, 2 * W
+                most = max(most, c * H * W)
+            prev = c
+        return max(most, ops.CONV_OUT_PAD * H * W)
+
+    def frames_per_group(self, h: int, w: int, max_launch_elements: int = MAX_LAUNCH_ELEMENTS) -> int:
+        per_frame = self.frame_elements(h, w)
+        if per_frame > max_launch_elements:
+            raise ValueError(f"one frame of a {h}x{w} latent needs {per_frame} elements in one launch "
+                             f"(limit {max_launch_elements}); decode it in tiles")
+        return max_launch_elements // per_frame
+
+    def _decode_group(self, zin, scale, as_uint8):
+        P = self._packed
+        N, _, h, w = zin.shape
         zq = ops.pointwise_conv_nchw(zin, P["pq"][0], P["pq"][1], scale)
         x = ops.conv_in(zq.reshape(N, 4, 1, h, w), P["conv_in"][0], P["conv_in"][1])
         H, W = h, w
         x = self._resnet("decoder.mid_block.resnets.0", x, N, H, W)
         x = self._attention(x, N, H * W)
         x = self._resnet("decoder.mid_block.resnets.1", x, N, H, W)
-        for i in range(len(UP_CHANNELS)):
-            for j in range(3):
+        levels = len(self.up_channels)
+        for i in range(levels):
+            for j in range(self.config.layers_per_block + 1):
                 x = self._resnet(f"decoder.up_blocks.{i}.resnets.{j}", x, N, H, W)
-            if i != len(UP_CHANNELS) - 1:
+            if i != levels - 1:
                 wu, bu, w4 = P[f"decoder.up_blocks.{i}.upsamplers.0.conv"]
                 if ops.upsample_conv3x3_supported(H, W, x.shape[1]):          # Upsample2D without the 4x copy
                     x = ops.upsample_conv3x3(x, N, H, W, w4, bias=bu, stats=True)
@@ -240,7 +298,29 @@ class VAEDecoder(nn.Module):
             hact = ops.groupnorm_apply(x, ss, N, H * W, True)
             y = ops.conv3x3(hact, N, H, W, P["conv_out"][0], bias=P["conv_out"][1], block_n=64, algo_n=3)
             return ops.image_to_uint8(y).reshape(N, H, W, 3)
-        out = ops.conv_out_tc(x, ss, N, 1, H, W, P["conv_out"][0], P["conv_out"][1], 3).reshape(N, 3, H, W)
+        return ops.conv_out_tc(x, ss, N, 1, H, W, P["conv_out"][0], P["conv_out"][1], 3).reshape(N, 3, H, W)
+
+    @torch.no_grad()
+    def decode(self, z: torch.Tensor, return_dict: bool = True, scale: float = 1.0, as_uint8: bool = False,
+               max_launch_elements: int = MAX_LAUNCH_ELEMENTS):
+        """AutoencoderKL.decode (mirror vsr/models/autoencoder_kl.py:179-198): z [N,4,h,w] -> ``.sample`` [N,3,sh,sw] in
+        z's dtype, s = 8 (SD VAE) or 4 (x4 upscaler).  ``scale`` multiplies z first (decode_latents' 1/scaling_factor);
+        ``as_uint8`` returns the pipelines' uint8 frames [N, sh, sw, 3] instead.  Frames run in groups of at most
+        ``frames_per_group(h, w, max_launch_elements)``; lowering the bound only regroups the same per-frame work."""
+        if z.dim() != 4 or z.shape[1] != 4:
+            raise ValueError(f"z must be [N,4,h,w], got {tuple(z.shape)}")
+        if self._packed is None:
+            self._pack()
+        dev = self.device
+        N, _, h, w = z.shape
+        zin = z.to(device=dev, dtype=F32).contiguous()
+        G = self.frames_per_group(h, w, max_launch_elements)
+        if N <= G:
+            out = self._decode_group(zin, scale, as_uint8)
+        else:
+            out = torch.cat([self._decode_group(zin[a:a + G], scale, as_uint8) for a in range(0, N, G)])
+        if as_uint8:
+            return out
         out = out.to(z.dtype) if z.dtype != F32 else out
         if not return_dict:
             return (out,)
@@ -248,9 +328,12 @@ class VAEDecoder(nn.Module):
 
     @torch.no_grad()
     def decode_latents(self, latents: torch.Tensor) -> torch.Tensor:
-        """VideoGenPipeline.decode_latents (base/pipelines/pipeline_videogen.py:422-429): [B,4,F,h,w] -> uint8
-        [B,F,H,W,3] on the host, with the 1/0.18215 scaling and the uint8 conversion inside the kernels."""
+        """The pipelines' decode_latents: [B,4,F,h,w] -> uint8 [B,F,sh,sw,3] on the host, with the 1/scaling_factor
+        scaling and the uint8 conversion inside the kernels.  SD VAE: VideoGenPipeline.decode_latents
+        (base/pipelines/pipeline_videogen.py:422-429); x4 upscaler: the VSR pipeline's decode
+        (vsr/models/pipeline_stable_diffusion_upscale_video_3d.py:741-771)."""
         B, C, Fr, h, w = latents.shape
         z = latents.permute(0, 2, 1, 3, 4).reshape(B * Fr, C, h, w)
-        video = self.decode(z, scale=1.0 / SCALING, as_uint8=True)
-        return video.reshape(B, Fr, 8 * h, 8 * w, 3).cpu().contiguous()
+        video = self.decode(z, scale=1.0 / self.config.scaling_factor, as_uint8=True)
+        s = self.upscale
+        return video.reshape(B, Fr, s * h, s * w, 3).cpu().contiguous()
