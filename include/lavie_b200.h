@@ -116,6 +116,16 @@ int lavie_conv3x3_supported(int H, int W, int C);
 int lavie_conv3x3_bf16(const void* x, int NF, int H, int W, int C, int stride, const void* w, void* out, int ldo, int N,
                        const lavie_epilogue* ep, int block_n, void* workspace, size_t workspace_bytes,
                        lavie_stream_t stream);
+/* The same conv with explicit zero padding: pad_before rows / columns before the image and pad_after after it, each 0
+ * or 1, on both axes.  (1, 1) is lavie_conv3x3_bf16; (0, 1) with stride 2 is diffusers' Downsample2D(padding=0), which
+ * pads (0, 1, 0, 1) and then runs a pad-0 conv: output pixel i reads input rows 2i, 2i+1, 2i+2.  The output has
+ * lavie_conv3x3_out_size(H, ...) x lavie_conv3x3_out_size(W, ...) pixels per image; the epilogue is unchanged. */
+int lavie_conv3x3_pad_bf16(const void* x, int NF, int H, int W, int C, int stride, int pad_before, int pad_after,
+                           const void* w, void* out, int ldo, int N, const lavie_epilogue* ep, int block_n,
+                           void* workspace, size_t workspace_bytes, lavie_stream_t stream);
+/* Output extent of a 3x3 conv along one axis of n pixels: (n + pad_before + pad_after - 3) / stride + 1, 0 when the
+ * padded extent is shorter than the filter.  Pure host query. */
+int lavie_conv3x3_out_size(int n, int stride, int pad_before, int pad_after);
 
 /* Patch matrix for the general / strided conv (Downsample3D stride 2, resnet.py:102-110):
  * col[NF*Ho*Wo, 9*C] with K ordered (kh, kw, c), pad 1. */
@@ -360,6 +370,17 @@ int lavie_pointwise_conv_nchw_f32(const float* x, const float* w, const float* b
 /* decode_latents post-processing (pipeline_videogen.py:426-428): out[pixel, 0..2] = uint8(clamp((y[pixel, 0..2] / 2 + 0.5)
  * * 255 + 0.5, 0, 255)); y bf16 channels-last rows of >= 4 columns. */
 int lavie_image_to_uint8(const void* y, int ld, long long pixels, unsigned char* out, lavie_stream_t stream);
+/* VAE encoder conv_in on uint8 video frames (the layout decode_latents returns): frames [N, H, W, 3] channels-last ->
+ * col bf16 [N*H*W, kpad], the rows lavie_im2col_input_bf16 writes for Cin = 3 from the normalised image
+ * (x / 255 - 0.5) / 0.5 (fp32, IEEE division); the conv is then lavie_gemm_bf16 against the [Cout, kpad] filters. */
+int lavie_im2col_frames_bf16(const unsigned char* frames, int N, int H, int W, int kpad, void* col,
+                             lavie_stream_t stream);
+/* AutoencoderKL.encode's DiagonalGaussianDistribution, sampled and scaled as the interpolation stage does
+ * (vae.encode(frames).latent_dist.sample().mul_(0.18215)): moments fp32 [B*F, 8, pixels] (mean | logvar, the quant_conv
+ * output), noise fp32 [B*F, 4, pixels] or NULL (then the mode, the mean, is taken) ->
+ * out fp32 [B, 4, F, pixels] = scale * (mean + exp(0.5 * clamp(logvar, -30, 20)) * noise), frame n = b * F + f. */
+int lavie_posterior_sample_f32(const float* moments, const float* noise, int B, int F, long long pixels, float scale,
+                               float* out, lavie_stream_t stream);
 
 /* ---------------------------------------------------------------------------------------------------------------
  * fp32-accumulate CHECK MODE (BASELINE north star: noise-prediction rel-L2 <= 1e-3 against the reference fp32 forward).

@@ -45,6 +45,9 @@ SIGNATURES = {
     "lavie_conv3x3_supported": (c_int, [c_int, c_int, c_int]),
     "lavie_conv3x3_bf16": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P, c_int, c_int, POINTER(Epilogue), c_int, _P,
                                    c_size_t, _P]),
+    "lavie_conv3x3_pad_bf16": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, c_int, c_int, _P, _P, c_int, c_int,
+                                       POINTER(Epilogue), c_int, _P, c_size_t, _P]),
+    "lavie_conv3x3_out_size": (c_int, [c_int, c_int, c_int, c_int]),
     "lavie_im2col3x3_bf16": (c_int, [_P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
     "lavie_groupnorm_chunks": (c_int, [c_int, c_int]),
     "lavie_groupnorm_stats": (c_int, [_P, c_int, c_int, _P, c_int, c_int, c_int, c_int, c_int, _P, _P]),
@@ -93,6 +96,8 @@ SIGNATURES = {
     "lavie_softmax_rows_bf16": (c_int, [_P, c_int, c_longlong, c_int, c_float, _P]),
     "lavie_attention_wide_bf16": (c_int, [_P, c_int, _P, c_int, _P, c_int, _P, c_int, c_int, c_int, _P]),
     "lavie_image_to_uint8": (c_int, [_P, c_int, c_longlong, _P, _P]),
+    "lavie_im2col_frames_bf16": (c_int, [_P, c_int, c_int, c_int, c_int, _P, _P]),
+    "lavie_posterior_sample_f32": (c_int, [_P, _P, c_int, c_int, c_longlong, c_float, _P, _P]),
     "lavie_pointwise_conv_nchw_f32": (c_int, [_P, _P, _P, c_float, c_int, c_int, c_int, c_longlong, _P, _P]),
     "lavie_groupnorm_finalize_colsums_seg": (c_int, [_P, c_int, c_int, _P, c_int, c_int, c_int, c_int, c_int, _P, _P,
                                                      c_float, _P, _P]),

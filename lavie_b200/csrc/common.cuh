@@ -30,7 +30,7 @@ int lavie_make_tmap(CUtensorMap* map, const void* base, int rank, const uint64_t
                     CUtensorMapSwizzle swizzle);
 
 int lavie_make_tmap_im2col(CUtensorMap* map, const void* base, int N, int H, int W, int C, int channels, int pixels,
-                           int stride, int corner_w = -1, int corner_h = -1);
+                           int stride, int lower_w, int lower_h, int upper_w, int upper_h);
 
 // ---------------------------------------------------------------------------------------------
 // Programmatic dependent launch (PDL): every kernel of the library is launched with

@@ -199,6 +199,31 @@ pointwise_conv_nchw_kernel(const float* __restrict__ x, const float* __restrict_
   }
 }
 
+// AutoencoderKL.encode's DiagonalGaussianDistribution and the interpolation stage's scaling
+// (interpolation/sample.py: vae.encode(frames).latent_dist.sample().mul_(0.18215)): moments fp32 [N, 8, pix] (mean |
+// logvar, as quant_conv leaves them) -> out[b, c, f, p] = scale * (mean + exp(0.5 * clamp(logvar, -30, 20)) * noise)
+// for frame n = b * F + f, i.e. the [B, 4, F, h, w] latents the interpolation UNet reads.  No noise: scale * mean.
+__global__ void __launch_bounds__(256)
+posterior_sample_kernel(const float* __restrict__ moments, const float* __restrict__ noise, int F, long long pix,
+                        long long total, float scale, float* __restrict__ out) {
+  pdl_prologue();
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const long long p = i % pix;
+    const long long nc = i / pix;                  // n * 4 + c
+    const int c = static_cast<int>(nc % 4);
+    const long long n = nc / 4;
+    const long long b = n / F;
+    const int f = static_cast<int>(n - b * F);
+    float z = moments[(n * 8 + c) * pix + p];
+    if (noise) {
+      const float lv = fminf(fmaxf(moments[(n * 8 + 4 + c) * pix + p], -30.0f), 20.0f);
+      z = z + expf(0.5f * lv) * noise[i];
+    }
+    out[((b * 4 + c) * F + f) * pix + p] = scale * z;
+  }
+}
+
 int grid_for_n(long long total, int threads) {
   long long b = (total + threads - 1) / threads;
   const long long cap = static_cast<long long>(lavie_num_sms()) * 16;
@@ -271,4 +296,13 @@ extern "C" int lavie_pointwise_conv_nchw_f32(const float* x, const float* w, con
   launch_pdl(pointwise_conv_nchw_kernel, grid_for_n(static_cast<long long>(N) * pixels, 256), 256, 0, stream, x, w, bias,
              scale, N, Cin, Cout, pixels, out);
   return lavie_check_launch("pointwise_conv_nchw_kernel");
+}
+
+extern "C" int lavie_posterior_sample_f32(const float* moments, const float* noise, int B, int F, long long pixels,
+                                          float scale, float* out, cudaStream_t stream) {
+  LAVIE_REQUIRE(moments && out && B > 0 && F > 0 && pixels > 0, LAVIE_ERR_SHAPE, "posterior_sample: bad arguments");
+  const long long total = static_cast<long long>(B) * F * 4 * pixels;
+  launch_pdl(posterior_sample_kernel, grid_for_n(total, 256), 256, 0, stream, moments, noise, F, pixels, total, scale,
+             out);
+  return lavie_check_launch("posterior_sample_kernel");
 }

@@ -61,6 +61,7 @@ struct GemmParams {
   int conv;                  // 0 plain GEMM, 1 implicit-GEMM 3x3 conv (im2col-mode TMA), 2 frame conv (k,1,1)
   int c_blocks;              // Cin / 64
   int out_h, out_w, conv_stride;   // im2col-mode conv (conv == 1): output geometry and stride
+  int pad_before;            // conv == 1: zero rows / columns before the image (1: pad (1, 1); 0: Downsample2D's (0, 1))
   int tap_rows;              // frame conv (conv == 2): rows between consecutive taps = pixels per frame
   int phases;                // 4: nearest-2x upsample + 3x3 conv as four 2x2 "phase" convs on the LOW-resolution map
                              // (conv == 3; item = (m, n, phase); output pixel (2y + py, 2x + px)); else 1
@@ -318,7 +319,8 @@ gemm_bf16_tcgen05(const __grid_constant__ CUtensorMap tmap_a0, const __grid_cons
               const int img = m0 / (p.out_h * p.out_w);
               const int rem = m0 - img * (p.out_h * p.out_w);
               const int oy = rem / p.out_w, ox = rem - oy * p.out_w;
-              tma2_load_im2col(a_dst, &tmap_a0, full_leader, c0, ox * p.conv_stride - 1, oy * p.conv_stride - 1, img,
+              tma2_load_im2col(a_dst, &tmap_a0, full_leader, c0, ox * p.conv_stride - p.pad_before,
+                               oy * p.conv_stride - p.pad_before, img,
                                static_cast<uint16_t>(tap % 3), static_cast<uint16_t>(tap / 3));
             } else if (kb < p.k_split_blocks) {
               tma2_load_2d(a_dst, &tmap_a0, full_leader, kb * BLOCK_K, m_cta * BLOCK_M);
@@ -1331,7 +1333,8 @@ extern "C" int lavie_upsample_conv3x3_bf16(const void* x, int NF, int H, int W, 
   if (rc) return rc;
   CUtensorMap ma[4], mb;
   for (int ph = 0; ph < 4; ++ph) {
-    rc = lavie_make_tmap_im2col(&ma[ph], x, NF, H, W, C, BLOCK_K, BLOCK_M, 1, (ph & 1) - 1, (ph >> 1) - 1);
+    rc = lavie_make_tmap_im2col(&ma[ph], x, NF, H, W, C, BLOCK_K, BLOCK_M, 1, (ph & 1) - 1, (ph >> 1) - 1, (ph & 1) - 1,
+                                (ph >> 1) - 1);
     if (rc) return rc;
   }
   // weights [4 phases * N, 4 * C]: phase-major rows, K ordered (a, b, c)
@@ -1352,23 +1355,33 @@ extern "C" int lavie_conv3x3_supported(int H, int W, int C) {
   return C % BLOCK_K == 0 ? 1 : 0;      // im2col-mode TMA handles any image geometry; channels come in 64-wide slabs
 }
 
+extern "C" int lavie_conv3x3_out_size(int n, int stride, int pad_before, int pad_after) {
+  const int padded = n + pad_before + pad_after;
+  return padded < 3 || stride < 1 ? 0 : (padded - 3) / stride + 1;
+}
+
 namespace {
-int conv3x3_impl(const void* x, int NF, int H, int W, int C, int stride, const void* w, void* out, int ldo, int N,
-                 const lavie_epilogue* ep, int block_n, void* workspace, size_t workspace_bytes, int check,
-                 cudaStream_t stream) {
+int conv3x3_impl(const void* x, int NF, int H, int W, int C, int stride, int pad_before, int pad_after, const void* w,
+                 void* out, int ldo, int N, const lavie_epilogue* ep, int block_n, void* workspace,
+                 size_t workspace_bytes, int check, cudaStream_t stream) {
   LAVIE_REQUIRE(lavie_conv3x3_supported(H, W, C), LAVIE_ERR_SHAPE, "conv3x3: C=%d must be a multiple of 64", C);
   LAVIE_REQUIRE(stride == 1 || stride == 2, LAVIE_ERR_SHAPE, "conv3x3: stride must be 1 or 2");
+  LAVIE_REQUIRE((pad_before == 0 || pad_before == 1) && (pad_after == 0 || pad_after == 1), LAVIE_ERR_SHAPE,
+                "conv3x3: padding (%d, %d) must be 0 or 1 on each side", pad_before, pad_after);
+  const int Ho = lavie_conv3x3_out_size(H, stride, pad_before, pad_after);
+  const int Wo = lavie_conv3x3_out_size(W, stride, pad_before, pad_after);
+  LAVIE_REQUIRE(Ho > 0 && Wo > 0, LAVIE_ERR_SHAPE, "conv3x3: H=%d W=%d too small for padding (%d, %d)", H, W, pad_before,
+                pad_after);
   LAVIE_REQUIRE(N % 8 == 0 && aligned16(x) && aligned16(w), LAVIE_ERR_ALIGN, "conv3x3: alignment");
   LAVIE_REQUIRE(workspace == nullptr || aligned16(workspace), LAVIE_ERR_ALIGN, "conv3x3: workspace alignment");
   LAVIE_REQUIRE(!(ep && ep->geglu), LAVIE_ERR_SHAPE, "conv3x3: GEGLU epilogue not supported");
-  const int Ho = (H - 1) / stride + 1, Wo = (W - 1) / stride + 1;
   const int M = NF * Ho * Wo;
   GemmParams p{};
   p.M = M; p.N = N; p.K = 9 * C;
   p.num_k_blocks = 9 * (C / BLOCK_K);
   p.k_split_blocks = p.num_k_blocks;
   p.c_blocks = C / BLOCK_K;
-  p.out_h = Ho; p.out_w = Wo; p.conv_stride = stride;
+  p.out_h = Ho; p.out_w = Wo; p.conv_stride = stride; p.pad_before = pad_before;
   p.conv = 1;
   p.check = check;
   int rc = check_workspace(check, M, N, workspace, workspace_bytes);
@@ -1378,7 +1391,8 @@ int conv3x3_impl(const void* x, int NF, int H, int W, int C, int stride, const v
   rc = fill_epilogue(p, ep, N, out, ldo);
   if (rc) return rc;
   CUtensorMap ma, mb;
-  rc = lavie_make_tmap_im2col(&ma, x, NF, H, W, C, BLOCK_K, BLOCK_M, stride);
+  rc = lavie_make_tmap_im2col(&ma, x, NF, H, W, C, BLOCK_K, BLOCK_M, stride, -pad_before, -pad_before, pad_after - 2,
+                              pad_after - 2);
   if (rc) return rc;
   rc = make_weight_map(&mb, w, N, 9 * C, plan.bn);
   if (rc) return rc;
@@ -1389,11 +1403,18 @@ int conv3x3_impl(const void* x, int NF, int H, int W, int C, int stride, const v
 extern "C" int lavie_conv3x3_bf16(const void* x, int NF, int H, int W, int C, int stride, const void* w, void* out,
                                   int ldo, int N, const lavie_epilogue* ep, int block_n, void* workspace,
                                   size_t workspace_bytes, cudaStream_t stream) {
-  return conv3x3_impl(x, NF, H, W, C, stride, w, out, ldo, N, ep, block_n, workspace, workspace_bytes, 0, stream);
+  return conv3x3_impl(x, NF, H, W, C, stride, 1, 1, w, out, ldo, N, ep, block_n, workspace, workspace_bytes, 0, stream);
+}
+
+extern "C" int lavie_conv3x3_pad_bf16(const void* x, int NF, int H, int W, int C, int stride, int pad_before,
+                                      int pad_after, const void* w, void* out, int ldo, int N, const lavie_epilogue* ep,
+                                      int block_n, void* workspace, size_t workspace_bytes, cudaStream_t stream) {
+  return conv3x3_impl(x, NF, H, W, C, stride, pad_before, pad_after, w, out, ldo, N, ep, block_n, workspace,
+                      workspace_bytes, 0, stream);
 }
 
 extern "C" int lavie_check_conv3x3(const void* x, int NF, int H, int W, int C3, int stride, const void* w, void* out,
                                    int ldo, int N, const lavie_epilogue* ep, void* workspace, size_t workspace_bytes,
                                    cudaStream_t stream) {
-  return conv3x3_impl(x, NF, H, W, C3, stride, w, out, ldo, N, ep, 0, workspace, workspace_bytes, 1, stream);
+  return conv3x3_impl(x, NF, H, W, C3, stride, 1, 1, w, out, ldo, N, ep, 0, workspace, workspace_bytes, 1, stream);
 }

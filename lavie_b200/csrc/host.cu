@@ -89,22 +89,24 @@ int lavie_make_tmap(CUtensorMap* map, const void* base, int rank, const uint64_t
   return LAVIE_OK;
 }
 
-// im2col-mode tensor map over a channels-last feature map [N, H, W, C] for a 3x3 pad-1 convolution: one TMA request
+// im2col-mode tensor map over a channels-last feature map [N, H, W, C] for a 3x3 convolution: one TMA request
 // fetches `pixels` consecutive OUTPUT pixels x `channels` input channels for one filter tap, walking the (W, H, N)
 // bounding box and zero-filling the halo (PTX ISA "im2col mode"; same corner convention as CUTLASS:
-// lower = -pad, upper = pad - (filter - 1)).
+// lower = -pad_before, upper = pad_after - (filter - 1)).  The box spans the filter windows' first input pixel, from
+// `lower` to (extent - 1 + upper), and is walked in steps of `stride`.
 int lavie_make_tmap_im2col(CUtensorMap* map, const void* base, int N, int H, int W, int C, int channels, int pixels,
-                           int stride, int corner_w, int corner_h) {
+                           int stride, int lower_w, int lower_h, int upper_w, int upper_h) {
   EncodeIm2colFn enc = get_encode_im2col();
   LAVIE_REQUIRE(enc != nullptr, LAVIE_ERR_DRIVER, "cuTensorMapEncodeIm2col is not available from the driver");
   const cuuint64_t gdim[4] = {static_cast<cuuint64_t>(C), static_cast<cuuint64_t>(W), static_cast<cuuint64_t>(H),
                               static_cast<cuuint64_t>(N)};
   const cuuint64_t gstr[3] = {static_cast<cuuint64_t>(C) * 2, static_cast<cuuint64_t>(W) * C * 2,
                               static_cast<cuuint64_t>(H) * W * C * 2};
-  // 3x3 pad 1: lower = upper = -1.  The 2x2 phase convs of the fused upsample (gemm.cu conv == 3) pad one pixel before
-  // (phase 0) or one pixel after (phase 1): lower = upper = phase - 1 per axis.
-  const int lower[2] = {corner_w, corner_h};
-  const int upper[2] = {corner_w, corner_h};
+  // 3x3 pad (1, 1): lower = upper = -1; Downsample2D's pad (0, 1): lower = 0, upper = -1.  The 2x2 phase convs of the
+  // fused upsample (gemm.cu conv == 3) pad one pixel before (phase 0) or one pixel after (phase 1): lower = upper =
+  // phase - 1 per axis.
+  const int lower[2] = {lower_w, lower_h};
+  const int upper[2] = {upper_w, upper_h};
   const cuuint32_t es[4] = {1, static_cast<cuuint32_t>(stride), static_cast<cuuint32_t>(stride), 1};
   CUresult r = enc(map, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), gdim, gstr, lower, upper,
                    static_cast<cuuint32_t>(channels), static_cast<cuuint32_t>(pixels), es, CU_TENSOR_MAP_INTERLEAVE_NONE,

@@ -364,6 +364,40 @@ im2col_input_kernel(const float* __restrict__ x, const float* __restrict__ input
   }
 }
 
+// The VAE encoder's conv_in on uint8 video frames (the layout decode_latents returns): channels-last [N, H, W, 3] ->
+// the same bf16 rows im2col_input_kernel writes for Cin = 3, with the interpolation stage's normalisation
+// (x / 255 - 0.5) / 0.5 evaluated in fp32 exactly as written (IEEE division: the library is built without fast-math).
+__global__ void __launch_bounds__(256)
+im2col_frames_kernel(const unsigned char* __restrict__ frames, int N, int H, int W, int kpad,
+                     __nv_bfloat16* __restrict__ col) {
+  pdl_prologue();
+  const int nvec = kpad >> 3;
+  const long long total = static_cast<long long>(N) * H * W * nvec;
+  const long long plane = static_cast<long long>(H) * W;
+  for (long long i = blockIdx.x * static_cast<long long>(blockDim.x) + threadIdx.x; i < total;
+       i += static_cast<long long>(gridDim.x) * blockDim.x) {
+    const int v = static_cast<int>(i % nvec);
+    const long long pix = i / nvec;
+    const int xo = static_cast<int>(pix % W);
+    const int yo = static_cast<int>((pix / W) % H);
+    const long long n = pix / plane;
+    float e[8];
+#pragma unroll
+    for (int j = 0; j < 8; ++j) {
+      const int k = v * 8 + j;
+      const int c = k / 9, tap = k - c * 9;
+      const int yy = yo + tap / 3 - 1, xx = xo + tap % 3 - 1;
+      e[j] = 0.f;
+      if (c < 3 && yy >= 0 && yy < H && xx >= 0 && xx < W) {
+        const float u = static_cast<float>(__ldg(frames + ((n * H + yy) * W + xx) * 3 + c));
+        e[j] = (u / 255.0f - 0.5f) / 0.5f;
+      }
+    }
+    *reinterpret_cast<uint4*>(col + pix * kpad + v * 8) =
+        make_uint4(pack_bf16(e[0], e[1]), pack_bf16(e[2], e[3]), pack_bf16(e[4], e[5]), pack_bf16(e[6], e[7]));
+  }
+}
+
 __global__ void cfg_ddim_kernel(const float* __restrict__ nu, const float* __restrict__ nt, float g, float sa_t,
                                 float s1a_t, float sa_p, float s1a_p, const float* __restrict__ lat,
                                 float* __restrict__ out, long long n) {
@@ -552,6 +586,17 @@ extern "C" int lavie_im2col_input_bf16(const float* x, const float* input_scale,
   launch_pdl(im2col_input_kernel, grid_for(total, 256), 256, 0, stream, x, input_scale, B, Cin, F, H, W, kpad,
              static_cast<__nv_bfloat16*>(col));
   return lavie_check_launch("im2col_input_kernel");
+}
+
+extern "C" int lavie_im2col_frames_bf16(const unsigned char* frames, int N, int H, int W, int kpad, void* col,
+                                        cudaStream_t stream) {
+  LAVIE_REQUIRE(frames && col && N > 0 && H > 0 && W > 0, LAVIE_ERR_SHAPE, "im2col_frames: bad arguments");
+  LAVIE_REQUIRE(kpad % 8 == 0 && kpad >= 27 && al16(col), LAVIE_ERR_SHAPE,
+                "im2col_frames: kpad=%d must be a multiple of 8 and >= 27, col 16-byte aligned", kpad);
+  const long long total = static_cast<long long>(N) * H * W * (kpad / 8);
+  launch_pdl(im2col_frames_kernel, grid_for(total, 256), 256, 0, stream, frames, N, H, W, kpad,
+             static_cast<__nv_bfloat16*>(col));
+  return lavie_check_launch("im2col_frames_kernel");
 }
 
 extern "C" int lavie_cfg_ddim_step(const float* noise_uncond, const float* noise_text, float guidance, float alpha_t,

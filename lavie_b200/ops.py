@@ -183,21 +183,31 @@ def im2col3x3(x: torch.Tensor, NF: int, H: int, W: int, stride: int = 1) -> torc
     return col
 
 
+def conv3x3_out_size(n: int, stride: int = 1, padding: Tuple[int, int] = (1, 1)) -> int:
+    """Output extent of a 3x3 conv along one axis of n pixels with ``padding`` = (before, after) zero pixels."""
+    return int(_lib.load().lavie_conv3x3_out_size(n, stride, padding[0], padding[1]))
+
+
 def conv3x3(x: torch.Tensor, NF: int, H: int, W: int, w: torch.Tensor, *, stride: int = 1, bias=None, row_bias=None,
             rows_per_batch=1, residual=None, out: Optional[torch.Tensor] = None, block_n: int = 0,
-            force_im2col: bool = False, stats: bool = False, algo_n: int = 0):
-    """3x3 pad-1 InflatedConv3d on a contiguous channels-last map; w: bf16 [N, 9*C] in (kh, kw, c) order.  ``algo_n``:
-    real output channels when the weight rows are zero-padded (launch accounting only)."""
+            force_im2col: bool = False, stats: bool = False, algo_n: int = 0, padding: Tuple[int, int] = (1, 1)):
+    """3x3 InflatedConv3d on a contiguous channels-last map; w: bf16 [N, 9*C] in (kh, kw, c) order.  ``algo_n``:
+    real output channels when the weight rows are zero-padded (launch accounting only).  ``padding`` = (before, after)
+    zero pixels on both axes: (1, 1) is the usual pad-1 conv, (0, 1) with stride 2 diffusers' Downsample2D(padding=0)."""
     lib = _lib.load()
     rows, C, ld = _rows2d(x)
     assert rows == NF * H * W and ld == C, "conv3x3 needs a contiguous channels-last input"
     N = w.shape[0]
     assert w.dtype == BF16 and w.is_contiguous() and w.shape[1] == 9 * C
+    pad_b, pad_a = (int(p) for p in padding)
     if force_im2col or not conv3x3_supported(H, W, C):
+        if (pad_b, pad_a) != (1, 1):
+            raise ValueError(f"conv3x3: the explicit im2col path only pads (1, 1), got padding={tuple(padding)} "
+                             f"(C={C}, force_im2col={force_im2col})")
         col = im2col3x3(x, NF, H, W, stride)
         return gemm(col, w, bias=bias, row_bias=row_bias, rows_per_batch=rows_per_batch, residual=residual, out=out,
                     block_n=block_n, stats=stats)
-    Ho, Wo = (H - 1) // stride + 1, (W - 1) // stride + 1
+    Ho, Wo = conv3x3_out_size(H, stride, (pad_b, pad_a)), conv3x3_out_size(W, stride, (pad_b, pad_a))
     m_out = NF * Ho * Wo
     if out is None:
         out = torch.empty((m_out, N), dtype=BF16, device=x.device)
@@ -207,12 +217,13 @@ def conv3x3(x: torch.Tensor, NF: int, H: int, W: int, w: torch.Tensor, *, stride
     ep = _epilogue(bias, row_bias, rows_per_batch, residual, False, cs)
     ws = _workspace(x.device)
     n_alg = algo_n or N
+    pad_tag = "" if (pad_b, pad_a) == (1, 1) else f" pad=({pad_b},{pad_a})"
     with _Launch("gemm_bf16_tcgen05", 2.0 * m_out * n_alg * 9 * C, 2.0 * (rows * C + n_alg * 9 * C + m_out * n_alg),
-                 f"conv3x3 M={m_out} N={N} K={9 * C} W={W} s={stride}"):
-        rc = lib.lavie_conv3x3_bf16(x.data_ptr(), NF, H, W, C, stride, w.data_ptr(), out.data_ptr(), ldo, N,
-                                    ctypes.byref(ep) if ep is not None else None, block_n, ws.data_ptr(),
-                                    ws.numel(), _stream())
-    check(rc, "lavie_conv3x3_bf16")
+                 f"conv3x3 M={m_out} N={N} K={9 * C} W={W} s={stride}{pad_tag}"):
+        rc = lib.lavie_conv3x3_pad_bf16(x.data_ptr(), NF, H, W, C, stride, pad_b, pad_a, w.data_ptr(), out.data_ptr(),
+                                        ldo, N, ctypes.byref(ep) if ep is not None else None, block_n, ws.data_ptr(),
+                                        ws.numel(), _stream())
+    check(rc, "lavie_conv3x3_pad_bf16")
     if cs is not None:
         out._gn_colsums = cs
     return out
