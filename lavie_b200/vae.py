@@ -31,11 +31,9 @@ from typing import Dict, Optional, Tuple
 import torch
 from torch import nn
 
-from . import ops
+from . import ops, vae_attention, vae_encode_ops
 from .packing import pack_conv1x1, pack_conv3x3, pack_upsample_conv3x3
 from .synthetic import _gen
-from .vae_attention import attention_wide
-from .vae_encode_ops import im2col_frames, posterior_sample
 
 BF16 = torch.bfloat16
 F32 = torch.float32
@@ -265,7 +263,7 @@ class _VAEModule(nn.Module):
         n = ops.groupnorm(x, N, HW, t["g"], t["b"], 1e-6, silu=False)
         if wide:
             qkv = ops.gemm(n, t["w_qkv"], bias=t["b_qkv"])                # [rows, 3C]; q already scaled by C^-1/2
-            o = attention_wide(qkv[:, :C], qkv[:, C:2 * C], qkv[:, 2 * C:], N, HW)
+            o = vae_attention.attention_wide(qkv[:, :C], qkv[:, C:2 * C], qkv[:, 2 * C:], N, HW)
             return ops.gemm(o, t["w_o"], bias=t["b_o"], residual=x, stats=True)
         if HW % 8:
             raise ValueError("the VAE mid-block attention needs h * w to be a multiple of 8")
@@ -468,7 +466,7 @@ class DiagonalGaussianDistribution:
         unless given."""
         N, _, h, w = self.parameters.shape
         eps = _noise_like((N, 4, h, w), generator, noise, self.parameters.device)
-        return posterior_sample(self.parameters, N, 1, 1.0, eps).reshape(N, 4, h, w)
+        return vae_encode_ops.posterior_sample(self.parameters, N, 1, 1.0, eps).reshape(N, 4, h, w)
 
     def mode(self) -> torch.Tensor:
         return self.mean
@@ -553,7 +551,7 @@ class VAEEncoder(_VAEModule):
         wi, bi = P["conv_in"]
         if frames:
             N, H, W, _ = x.shape
-            h = ops.gemm(im2col_frames(x, wi.shape[1]), wi, bias=bi)
+            h = ops.gemm(vae_encode_ops.im2col_frames(x, wi.shape[1]), wi, bias=bi)
         else:
             N, _, H, W = x.shape
             h = ops.conv_in_tc(x.reshape(N, 3, 1, H, W), wi, bi)
@@ -613,4 +611,5 @@ class VAEEncoder(_VAEModule):
         if self._packed is None:
             self._pack()
         fr = frames.to(dev).reshape(B * Fr, H, W, 3).contiguous()
-        return posterior_sample(self._moments(fr, True, max_launch_elements), B, Fr, self.config.scaling_factor, eps)
+        return vae_encode_ops.posterior_sample(self._moments(fr, True, max_launch_elements), B, Fr,
+                                               self.config.scaling_factor, eps)

@@ -1,8 +1,9 @@
 """Per-launch audit: every kernel launch the denoisers and encoders issue, checked against a high-precision reference of
 that one launch.
 
-A recorder wraps the launching functions of `lavie_b200.ops` (all model code calls through the module attribute), clones
-each call's tensor arguments before the call (outputs alias inputs: `out=` views, residual/out pairs, in-place ops), runs
+A recorder wraps the launching functions of the launch modules (`lavie_b200.ops`, and the modules that keep the VAE's own
+launches: `vae_attention`, `vae_encode_ops`), which model code calls through the module attribute (a CPU test parses the
+model files to hold that), clones each call's tensor arguments before the call (outputs alias inputs: `out=` views, residual/out pairs, in-place ops), runs
 the real function on the original tensors and compares the result, right away, with a reference computed in fp64 from
 the cloned inputs.  Only a summary row per launch is kept.
 
@@ -12,10 +13,13 @@ ones, a key-index ramp) that a mask off by one key moves by more than the bound.
 bytes around `out=` views are checked too.  The comparators are plain torch: the CPU tests at the end inject defects into
 a correct bf16 result and show that each is flagged, and that an uninjected result passes.
 """
+import ast
 import collections
+import importlib
 import inspect
 import math
 import os
+import re
 import sys
 
 import pytest
@@ -188,23 +192,62 @@ def geglu_ref(h, s, c):
     return ref, extra
 
 
-def im2col64(x, NF, H, W, stride=1):
-    """x [NF*H*W, C] -> [NF*Ho*Wo, 9*C] in fp64, K ordered (kh, kw, c), zero padding 1."""
+def conv_out_size(n, stride=1, padding=(1, 1)):
+    """Output extent of a 3x3 conv along n pixels with (before, after) zero padding: the formula of
+    ops.conv3x3_out_size (lavie_conv3x3_out_size)."""
+    p = n + padding[0] + padding[1]
+    return 0 if p < 3 else (p - 3) // stride + 1
+
+
+def im2col64(x, NF, H, W, stride=1, padding=(1, 1), lines=None):
+    """x [NF*H*W, C] -> [NF*Ho*Wo, 9*C] in fp64, K ordered (kh, kw, c), `padding` = (before, after) zero pixels on both
+    axes; `lines` = (y0, y1): only those output lines of every image."""
     C = x.shape[1]
-    Ho, Wo = (H - 1) // stride + 1, (W - 1) // stride + 1
-    xp = F.pad(x.to(F64).reshape(NF, H, W, C), (0, 0, 1, 1, 1, 1))
-    taps = [xp[:, kh:kh + stride * (Ho - 1) + 1:stride, kw:kw + stride * (Wo - 1) + 1:stride] for kh in range(3)
+    pb, pa = padding
+    Ho, Wo = conv_out_size(H, stride, padding), conv_out_size(W, stride, padding)
+    y0, y1 = lines or (0, Ho)
+    top, bot = y0 * stride - pb, (y1 - 1) * stride - pb + 3            # input lines the band reads, end exclusive
+    band = x.reshape(NF, H, W, C)[:, max(top, 0):min(bot, H)].to(F64)
+    xp = F.pad(band, (0, 0, pb, pa, max(0, -top), max(0, bot - H)))
+    n = y1 - y0
+    taps = [xp[:, kh:kh + stride * (n - 1) + 1:stride, kw:kw + stride * (Wo - 1) + 1:stride] for kh in range(3)
             for kw in range(3)]
-    return torch.stack(taps, 3).reshape(NF * Ho * Wo, 9 * C)
+    return torch.stack(taps, 3).reshape(NF * n * Wo, 9 * C)
 
 
-def conv_mm(x, NF, H, W, stride, w):
-    """3x3 pad-1 conv of x [NF*H*W, C] with w [N, 9*C] ((kh, kw, c) order) and its abs-product, chunked over images."""
-    Ho, Wo = (H - 1) // stride + 1, (W - 1) // stride + 1
-    imgs = max(1, (1 << 27) // (Ho * Wo * w.shape[1]))
+def conv_rows(x, NF, H, W, stride=1, padding=(1, 1)):
+    """rows(lo, hi) -> rows lo..hi of the conv's fp64 patch matrix (lo, hi on output-line boundaries), built image by image
+    or, inside one image, line band by line band."""
+    Ho, Wo = conv_out_size(H, stride, padding), conv_out_size(W, stride, padding)
     o, hw = Ho * Wo, H * W
-    return mm_abs(lambda lo, hi: im2col64(x[lo // o * hw:hi // o * hw], (hi - lo) // o, H, W, stride), w,
-                  rows=NF * o, step=imgs * o)
+
+    def rows(lo, hi):
+        if lo % o == 0 and hi % o == 0:
+            return im2col64(x[lo // o * hw:hi // o * hw], (hi - lo) // o, H, W, stride, padding)
+        parts = []
+        while lo < hi:
+            n = lo // o
+            e = min(hi, (n + 1) * o)
+            parts.append(im2col64(x[n * hw:(n + 1) * hw], 1, H, W, stride, padding,
+                                  ((lo - n * o) // Wo, (e - n * o + Wo - 1) // Wo)))
+            lo = e
+        return torch.cat(parts)
+    return rows
+
+
+def conv_step(Ho, Wo, width):
+    """Rows per comparison block of a conv output: whole images when one fits Cmp.STEP patch elements, else bands of
+    whole output lines."""
+    o = Ho * Wo
+    if o * width <= Cmp.STEP:
+        return max(1, Cmp.STEP // (width * o)) * o
+    return max(1, Cmp.STEP // (width * Wo)) * Wo
+
+
+def conv_mm(x, NF, H, W, stride, w, padding=(1, 1)):
+    """3x3 conv of x [NF*H*W, C] with w [N, 9*C] ((kh, kw, c) order) and its abs-product, in blocks of conv_step rows."""
+    Ho, Wo = conv_out_size(H, stride, padding), conv_out_size(W, stride, padding)
+    return mm_abs(conv_rows(x, NF, H, W, stride, padding), w, rows=NF * Ho * Wo, step=conv_step(Ho, Wo, w.shape[1]))
 
 
 def upsample_phase_ref(x, NF, H, W, w_phases):
@@ -482,12 +525,11 @@ def _img_step(per_img, width):
 
 
 def chk_conv3x3(a, res, ctx):
-    NF, H, W, s_ = a["NF"], a["H"], a["W"], a["stride"]
-    Ho, Wo = (H - 1) // s_ + 1, (W - 1) // s_ + 1
-    x, o, hw = a["x"], Ho * Wo, H * W
-    cmp = gemm_check(res, lambda lo, hi: im2col64(x[lo // o * hw:hi // o * hw], (hi - lo) // o, H, W, s_), a["w"],
-                     a["w"].shape[1], a, ctx.get("splits", 1), step=_img_step(o, a["w"].shape[1]),
-                     dims=("image", "y", "x", "channel"))
+    NF, H, W, s_, pad = a["NF"], a["H"], a["W"], a["stride"], tuple(a["padding"])
+    Ho, Wo = conv_out_size(H, s_, pad), conv_out_size(W, s_, pad)
+    o = Ho * Wo
+    cmp = gemm_check(res, conv_rows(a["x"], NF, H, W, s_, pad), a["w"], a["w"].shape[1], a, ctx.get("splits", 1),
+                     step=conv_step(Ho, Wo, a["w"].shape[1]), dims=("image", "y", "x", "channel"))
     r, c = cmp.worst_at
     cmp.worst_at = (r // o, r // Wo % Ho, r % Wo, c)
     return [cmp]
@@ -800,7 +842,116 @@ def chk_pointwise_conv_nchw(a, res, ctx):
     return [Cmp("pointwise_conv_nchw", res, ref, (x.shape[1] + 2) * U32 * mag + 1e-300)]
 
 
-CHECKERS = {
+def frame_values():
+    """bf16 (u / 255 - 0.5) / 0.5 for u = 0..255, divided in numpy fp32 (IEEE, as the kernel divides).  Not torch on the
+    GPU: its division by a scalar multiplies by the fp32 reciprocal, which puts u = 127 on the neighbouring bf16."""
+    import numpy as np
+    u = np.arange(256, dtype=np.float32)
+    return torch.from_numpy((u / np.float32(255) - np.float32(0.5)) / np.float32(0.5)).to(BF16)
+
+
+def chk_im2col_frames(a, res, ctx):
+    """The kernel's contract (vae_encode_ops.im2col_frames): (x / 255 - 0.5) / 0.5 in fp32, rounded to bf16 once, K index
+    c*9 + kh*3 + kw, zero outside the image and in the K columns 27..kpad.  Exact."""
+    fr = a["frames"]
+    N, H, W, _ = fr.shape
+    x = frame_values()[fr.long().cpu()].to(fr.device).permute(0, 3, 1, 2).to(F64)
+    ref = torch.zeros((N * H * W, a["kpad"]), dtype=F64, device=fr.device)
+    ref[:, :27] = F.unfold(x, 3, padding=1).transpose(1, 2).reshape(N * H * W, 27)
+    cmp = Cmp("im2col_frames", res, ref, 1e-300, dims=("frame", "y", "x", "column"))
+    r, c = cmp.worst_at
+    cmp.worst_at = (r // (H * W), r // W % H, r % W, c)
+    return [cmp]
+
+
+def posterior_ref(moments, B, F_, scale, noise):
+    """scale * (mean + exp(0.5 clamp(logvar, -30, 20)) noise) in fp64 in the [B, 4, F, h, w] layout (noise None: the
+    mode, scale * mean), and its bound: fp32 exp (2 ulp), the fma and the scaling (one rounding each) and the fp32 scale
+    stay within 2^-20 of scale (|mean| + std |noise|)."""
+    m = moments.to(F64)
+    mean = m[:, :4]
+    ref, mag = mean, mean.abs()
+    if noise is not None:
+        std = torch.exp(0.5 * m[:, 4:].clamp(-30, 20))
+        ref = mean + std * noise.to(F64)
+        mag = mag + std * noise.to(F64).abs()
+    N, _, h, w = moments.shape
+    lay = lambda t: t.reshape(B, F_, 4, h, w).permute(0, 2, 1, 3, 4)          # noqa: E731
+    return lay(scale * ref), lay(2.0 ** -20 * abs(scale) * mag + 1e-30)
+
+
+def chk_posterior_sample(a, res, ctx):
+    ref, bnd = posterior_ref(a["moments"], a["B"], a["F"], a["scale"], a["noise"])
+    return [Cmp("posterior_sample", res, ref, bnd, None, ("item", "channel", "frame", "y", "x"))]
+
+
+# attention_wide (one head, d = 512, q pre-scaled): the score Q K^T is a tcgen05 GEMM over K = 512, so its error is the
+# GEMM's accumulation bound c_gemm(512) = 41 * 2^-23 (~2^-17.6) of each key's sum |q| |k|; the 9 split / epilogue terms
+# the score does not use cover the fp32 exp2 argument (s log2 e - m: < 3 roundings of |s| <= sum |q| |k|).  P is rounded
+# to bf16 for P V while the row sum adds the unrounded p, so o moves by at most 2^-9 sum p |v| <= U sum p |v| (C_ATTN_P
+# keeps another U for the other attention kernels; the x4 kernel tests have always used U here).  Each of the three fp32
+# chains over a frame's S keys -- P V accumulated in TMEM (ceil(S/16) MMA steps), the row sum (S/64 tile sums of 32
+# terms) and the O / row-sum rescales of the lazy maximum (at most one per 64-key tile) -- stays within c_gemm(S) of
+# sum p |v|.  tests/test_vae_x4_gpu.py checks the kernel against this same bound; the one it had before took 2^-15 of
+# the row's largest sum |q| |k| for every key (6x RHO_WIDE) and S 2^-23 for the chains (over 5x 3 c_gemm(S)).
+RHO_WIDE = c_gemm(512)
+WIDE_D = 512
+WIDE_FULL_S = 16384     # above this many tokens per frame the reference covers a sample of query rows (wide_query_rows)
+
+
+def c_attn_wide(S):
+    return U + 3 * c_gemm(S)
+
+
+def wide_query_rows(S):
+    """None (every row) up to WIDE_FULL_S tokens, else a deterministic sample of query rows (indices within a frame): the
+    first and the last 128-query tile, the rows on both sides of 16 tile boundaries spread over the frame, and up to 1024
+    rows drawn with a fixed seed."""
+    if S <= WIDE_FULL_S:
+        return None
+    last = (S - 1) // 128 * 128
+    picks = [torch.arange(0, 128), torch.arange(last, S)]
+    for t in torch.linspace(1, last // 128, 16).long().unique().tolist():
+        picks.append(torch.arange(t * 128 - 2, t * 128 + 2))
+    picks.append(torch.randperm(S, generator=torch.Generator().manual_seed(S))[:min(1024, S // 8)])
+    return torch.cat(picks).unique()
+
+
+def wide_attention_ref(q, k, v, frames, S, rows=None):
+    """softmax(q k^T) v per frame in fp64 and its bound (attention_core: frames as the batch, one head, scale 1 since q
+    carries 512^-1/2); rows: only these query rows of every frame.  Returns [frames, rows or S, 512]."""
+    Q, K, V = (t.reshape(frames, 1, S, WIDE_D) for t in (q, k, v))
+    if rows is not None:
+        Q = Q[:, :, rows.to(q.device)]
+    o, bnd = attention_core(Q, K, V, 1.0, rho=RHO_WIDE, c_p=c_attn_wide(S))
+    return o[:, 0], bnd[:, 0]
+
+
+def _wide_cmp(what, got, a, rows, ref, bnd, cols=None):
+    frames, S = a["frames"], a["S"]
+    g = got.reshape(frames, S, WIDE_D)
+    if rows is not None:
+        g = g[:, rows.to(g.device)]
+    if cols is not None:
+        g, ref, bnd = g[..., cols], ref[..., cols], bnd[..., cols]
+    cmp = Cmp(what, g, ref, bnd, REL_ATTN if cols is None else None, ("frame", "query", "column"))
+    if rows is not None:
+        f, i, c = cmp.worst_at
+        cmp.worst_at = (f, int(rows[i]), c)
+    return cmp
+
+
+def chk_attention_wide(a, res, ctx):
+    rows = wide_query_rows(a["S"])
+    ref, bnd = wide_attention_ref(a["q"], a["k"], a["v"], a["frames"], a["S"], rows)
+    out = [_wide_cmp("attention_wide" + (" (sampled rows)" if rows is not None else ""), res, a, rows, ref, bnd)]
+    if ctx.get("probe") is not None:
+        out += ctx["probe"](a, res)
+    return out
+
+
+# (module, function) -> checker: the recorder wraps each function in the module it lives in
+CHECKERS = {("ops", n): f for n, f in {
     "gemm": chk_gemm, "conv3x3": chk_conv3x3, "im2col3x3": chk_im2col3x3, "frame_conv": chk_frame_conv,
     "upsample_conv3x3": chk_upsample_conv3x3, "groupnorm_scale_shift": chk_groupnorm_scale_shift,
     "groupnorm_apply": chk_groupnorm_apply, "groupnorm": chk_groupnorm, "layernorm": chk_layernorm,
@@ -812,35 +963,83 @@ CHECKERS = {
     "cfg_linear_step": chk_cfg_linear_step, "cfg_combine": chk_cfg_combine, "clip_embed": chk_clip_embed,
     "activation_": chk_activation_, "softmax_rows_": chk_softmax_rows_, "image_to_uint8": chk_image_to_uint8,
     "pointwise_conv_nchw": chk_pointwise_conv_nchw,
+}.items()}
+CHECKERS.update({
+    ("vae_attention", "attention_wide"): chk_attention_wide,
+    ("vae_encode_ops", "im2col_frames"): chk_im2col_frames,
+    ("vae_encode_ops", "posterior_sample"): chk_posterior_sample,
+})
+
+_P2P_SOLO = "tests/test_p2p_gpu.py::test_p2p_kernels_with_a_single_peer"
+_CHECK_MODELS = ("tests/test_check_mode_gpu.py::test_matches_reference_golden_check, "
+                 "tests/test_check_mode_gpu.py::test_interp_check_mode (check-mode model runs)")
+# launching functions that the model runs below do not issue, with the test that covers each
+COVERED_ELSEWHERE = {
+    ("ops", "layernorm_scatter"): "tests/test_sharding_gpu.py, tests/test_p2p_gpu.py (frame-sharded temporal attention)",
+    ("ops", "add_gathered"): "tests/test_sharding_gpu.py, tests/test_p2p_gpu.py (frame-sharded temporal attention)",
+    ("ops", "groupnorm_sums"): "tests/test_sharding_gpu.py (frame-sharded GroupNorm statistics)",
+    ("ops", "groupnorm_finalize_sums"): "tests/test_sharding_gpu.py (frame-sharded GroupNorm statistics)",
+    ("ops", "conv_out"): "tests/test_kernels_gpu.py::test_conv_in_and_out (fp32 conv_out, used when C % 64 != 0)",
+    ("ops", "im2col3x3"): "tests/test_kernels_gpu.py::test_conv3x3_stride_and_explicit_im2col (explicit patch matrix, "
+                          "C % 64 != 0)",
+    # peer-memory frame sharding (one GPU as its own peer; two GPUs against the un-sharded forward)
+    ("p2p", "PeerContext.push_halo"): _P2P_SOLO,
+    ("p2p", "PeerContext.gn_scale_shift"): _P2P_SOLO,
+    ("p2p", "PeerContext.layernorm_scatter"): _P2P_SOLO + ", tests/test_sharding_gpu.py",
+    ("p2p", "PeerContext.add_gathered"): _P2P_SOLO + ", tests/test_sharding_gpu.py",
+    ("p2p", "PeerContext.barrier"): "tests/test_p2p_gpu.py::test_two_gpu_frame_sharding_matches_single_gpu",
+    # the fp32-accumulate check mode (split-bf16 triples), against fp64 kernel by kernel and the reference's fp32 forward
+    ("check", "gemm"): "tests/test_check_mode_gpu.py::test_check_gemm_epilogues",
+    ("check", "conv3x3"): "tests/test_check_mode_gpu.py::test_check_conv3x3",
+    ("check", "groupnorm_scale_shift"): "tests/test_check_mode_gpu.py::test_check_norms",
+    ("check", "groupnorm_apply"): "tests/test_check_mode_gpu.py::test_check_norms",
+    ("check", "groupnorm"): "tests/test_check_mode_gpu.py::test_check_norms",
+    ("check", "layernorm"): "tests/test_check_mode_gpu.py::test_check_norms",
+    ("check", "attention"): "tests/test_check_mode_gpu.py::test_check_attention",
+    ("check", "temporal_attention"): _CHECK_MODELS,
+    ("check", "frame_attention"): _CHECK_MODELS,
+    ("check", "text_input"): _CHECK_MODELS,
+    ("check", "linear_smallm"): _CHECK_MODELS,
+    ("check", "conv_in"): _CHECK_MODELS,
+    ("check", "conv_out"): _CHECK_MODELS,
 }
 
-# launching functions of `ops` that the model runs below do not issue, with the test that covers each
-COVERED_ELSEWHERE = {
-    "layernorm_scatter": "tests/test_sharding_gpu.py, tests/test_p2p_gpu.py (frame-sharded temporal attention)",
-    "add_gathered": "tests/test_sharding_gpu.py, tests/test_p2p_gpu.py (frame-sharded temporal attention)",
-    "groupnorm_sums": "tests/test_sharding_gpu.py (frame-sharded GroupNorm statistics)",
-    "groupnorm_finalize_sums": "tests/test_sharding_gpu.py (frame-sharded GroupNorm statistics)",
-    "conv_out": "tests/test_kernels_gpu.py::test_conv_in_and_out (fp32 conv_out, used when C % 64 != 0)",
-    "im2col3x3": "tests/test_kernels_gpu.py::test_conv3x3_stride_and_explicit_im2col (explicit patch matrix, C % 64 != 0)",
-}
+PKG = os.path.join(os.path.dirname(os.path.dirname(os.path.abspath(__file__))), "lavie_b200")
+
+
+def launch_modules():
+    """The modules of lavie_b200 that launch kernels: every lavie_b200/*.py whose source issues a `_Launch(`."""
+    mods = []
+    for fn in sorted(os.listdir(PKG)):
+        if fn.endswith(".py"):
+            with open(os.path.join(PKG, fn)) as f:
+                if "_Launch(" in f.read():
+                    mods.append(fn[:-3])
+    return mods
 
 
 def launching_functions():
-    """Every public function of `ops` that launches a kernel itself or through another one."""
-    from lavie_b200 import ops
-    names = set()
-    for name, fn in inspect.getmembers(ops, inspect.isfunction):
-        if fn.__module__ != ops.__name__ or name.startswith("_"):
-            continue
-        src = inspect.getsource(fn)
-        if "_Launch(" in src:
-            names.add(name)
-    for name, fn in inspect.getmembers(ops, inspect.isfunction):       # composites: call a launching function
-        if fn.__module__ == ops.__name__ and not name.startswith("_") and name not in names:
-            src = inspect.getsource(fn).split(":", 1)[1]
-            if any(f"{n}(" in src for n in names if n != name):
-                names.add(name)
-    return names
+    """(module, name) of every public function of a launch module -- and every public method of its classes, named
+    Class.method -- that launches a kernel itself or through another one (private helpers included)."""
+    out = set()
+    for modname in launch_modules():
+        mod = importlib.import_module(f"lavie_b200.{modname}")
+        fns = {n: f for n, f in inspect.getmembers(mod, inspect.isfunction) if f.__module__ == mod.__name__}
+        for cname, cls in inspect.getmembers(mod, inspect.isclass):
+            if cls.__module__ == mod.__name__:
+                fns.update({f"{cname}.{m}": f for m, f in vars(cls).items() if inspect.isfunction(f)})
+        src = {n: inspect.getsource(f) for n, f in fns.items()}
+        names = {n for n in fns if "_Launch(" in src[n]}
+        grown = True
+        while grown:                                    # composites: call a launching function (or method)
+            grown = False
+            for n in fns:
+                if n not in names and any(re.search(rf"\b{re.escape(c.rsplit('.', 1)[-1])}\(", src[n])
+                                          for c in names if c != n):
+                    names.add(n)
+                    grown = True
+        out |= {(modname, n) for n in names if not n.rsplit(".", 1)[-1].startswith("_")}
+    return out
 
 
 def ramp_values(rows, seq_len, seq_stride, F_=None):
@@ -858,6 +1057,8 @@ def attention_probes(name, real, a):
     column (every output must be 1 within 2^-7: an extra or missing key or a wrong normalisation moves it by ~1/keys),
     then V = key-index ramps (ramp_values) in the first columns of every head, whose outputs must match the fp64
     expected key index within the attention bound."""
+    if name == "attention_wide":
+        return wide_attention_probes(real, a)
     heads, d, pitch = a["heads"], a["d"], a["head_pitch"]
     out = []
     for kind in ("ones", "ramp"):
@@ -905,8 +1106,35 @@ def attention_probes(name, real, a):
     return out
 
 
+def wide_attention_probes(real, a):
+    """attention_probes for attention_wide: V = 1 in all 512 columns, then the key-index ramps (position in the frame,
+    position mod 64, frame mod 64) in columns 0..2, on the rows of wide_query_rows."""
+    frames, S = a["frames"], a["S"]
+    rows = wide_query_rows(S)
+    q, k = a["q"], a["k"]
+    out = []
+    for kind in ("ones", "ramp"):
+        v = torch.zeros((frames * S, WIDE_D), dtype=BF16, device=k.device)
+        if kind == "ones":
+            v.fill_(1.0)
+        else:
+            v[:, :3] = ramp_values(frames * S, S, 1).to(device=k.device, dtype=BF16)
+        got = real(q, k, v, frames, S)
+        if got.is_cuda:
+            torch.cuda.synchronize()
+        if kind == "ones":
+            g = got.reshape(frames, S, WIDE_D)
+            g = g if rows is None else g[:, rows.to(g.device)]
+            out.append(Cmp("attention_wide probe V=1", g, torch.ones((), dtype=F64), 2.0 ** -7))
+        else:
+            ref, bnd = wide_attention_ref(q, k, v, frames, S, rows)
+            out.append(_wide_cmp("attention_wide probe V=key ramp", got, a, rows, ref, bnd, cols=slice(0, 3)))
+    return out
+
+
 # ------------------------------------------------------------------------------------------------ recorder
 MODEL_FILES = ("unet.py", "vsr.py", "vae.py", "clip.py")
+PROBED = ("attention", "frame_attention", "temporal_attention", "attention_wide")
 
 
 def model_block():
@@ -956,7 +1184,7 @@ class OpRow:
 
 
 class Recorder:
-    """Wraps the launching functions of `ops` for the duration of a `with` block."""
+    """Wraps the checked launching functions (CHECKERS) in their modules for the duration of a `with` block."""
 
     def __init__(self, log):
         from lavie_b200 import _lib, ops
@@ -969,15 +1197,16 @@ class Recorder:
 
     def __enter__(self):
         self.tf32 = tf32_off()
-        for name in CHECKERS:
-            fn = getattr(self.ops, name)
-            self.real[name] = fn
-            setattr(self.ops, name, self._wrap(name, fn))
+        for (modname, name), check in CHECKERS.items():
+            mod = importlib.import_module(f"lavie_b200.{modname}")
+            fn = getattr(mod, name)
+            self.real[name] = (mod, fn)
+            setattr(mod, name, self._wrap(name, fn, check))
         return self
 
     def __exit__(self, *exc):
-        for name, fn in self.real.items():
-            setattr(self.ops, name, fn)
+        for name, (mod, fn) in self.real.items():
+            setattr(mod, name, fn)
         tf32_restore(self.tf32)
         return False
 
@@ -992,9 +1221,8 @@ class Recorder:
             kinds.add("main+tail window")
         return kinds, max(sp.value, ts.value, 1)
 
-    def _wrap(self, name, fn):
+    def _wrap(self, name, fn, check):
         sig = inspect.signature(fn)
-        check = CHECKERS[name]
 
         def wrapper(*args, **kw):
             bound = sig.bind(*args, **kw)
@@ -1020,11 +1248,13 @@ class Recorder:
                 elif name == "conv3x3":
                     K = a["w"].shape[1]
                     plans, splits = self._plan(res.shape[0], a["w"].shape[0], K, 1, False)
+                    if tuple(a["padding"]) != (1, 1):
+                        plans.add("pad ({},{})".format(*a["padding"]))
                 else:
                     K = a["w"].shape[1]
                     plans, splits = self._plan(res.shape[0], a["w"].shape[0], K, 0, False)
                 ctx["splits"] = splits
-            if name in ("attention", "frame_attention", "temporal_attention"):
+            if name in PROBED:
                 key = (name,) + tuple((k, tuple(v.shape) if torch.is_tensor(v) else v) for k, v in a.items()
                                       if k not in ("out", "scale"))
                 if key not in self.probed:
@@ -1048,7 +1278,7 @@ class Recorder:
         return wrapper
 
     def _probe(self, name, a, res):
-        return attention_probes(name, self.real[name], a)
+        return attention_probes(name, self.real[name][1], a)
 
     def _record(self, name, idx, block, a, results, plans, probed):
         row = self.log.rows[name]
@@ -1061,7 +1291,7 @@ class Recorder:
             if not r.ok:
                 shapes = {k: (tuple(v.shape) if torch.is_tensor(v) else v) for k, v in a.items()
                           if torch.is_tensor(v) or isinstance(v, (int, float, bool, str))}
-                self.log.failures.append(f"[{self.log.run}] #{idx} ops.{name} from {block}: {r}; args {shapes}"
+                self.log.failures.append(f"[{self.log.run}] #{idx} {name} from {block}: {r}; args {shapes}"
                                          + (f"; plan {sorted(plans)}" if plans else ""))
 
 
@@ -1088,7 +1318,7 @@ class AuditLog:
 
 # ------------------------------------------------------------------------------------------------ GPU runs
 RUNS_DEFAULT = ("base headline", "base ragged", "interpolation 61f", "vsr 16f", "vsr ragged", "clip", "vae 40x64",
-                "vae ragged")
+                "vae ragged", "vae encoder", "vae encoder ragged", "vae x4", "vae x4 ragged")
 
 
 @pytest.fixture(scope="session")
@@ -1270,30 +1500,140 @@ def test_audit_vae_ragged_uint8(vae, audit_log, reference_selfcheck):
     _finish(audit_log)
 
 
+@pytest.fixture(scope="module")
+def vae_encoder():
+    from lavie_b200.vae import VAEEncoder, vae_encoder_synthetic_state_dict
+    m = VAEEncoder()
+    m.load_state_dict(vae_encoder_synthetic_state_dict(seed=0), strict=True)
+    return m.to("cuda").eval()
+
+
+def _video(B, Fr, H, W, seed):
+    return torch.randint(0, 256, (B, Fr, H, W, 3), dtype=torch.uint8, generator=torch.Generator().manual_seed(seed))
+
+
+@pytest.mark.gpu
+def test_audit_vae_encoder_production_frames(vae_encoder, audit_log, reference_selfcheck):
+    """The interpolation stage's encode: 2 uint8 frames of 320x512 (40x64 latent) with fixed noise: patch rows straight
+    from the frames, the stride-2 pad (0, 1) downsample convs with producer statistics, the mid-block attention,
+    conv_out on the tensor cores, quant_conv and the posterior sample."""
+    g = torch.Generator().manual_seed(320)
+    noise = torch.randn(2, 4, 40, 64, generator=g)
+    with audit_log.record("vae encoder"):
+        vae_encoder.encode_video(_video(1, 2, 320, 512, 1).cuda(), noise=noise.cuda())
+    _finish(audit_log)
+
+
+@pytest.mark.gpu
+def test_audit_vae_encoder_ragged(vae_encoder, audit_log, reference_selfcheck):
+    """3 frames of 56x128 (7x16 latent: 112 rows per frame, so the GroupNorms fall back to the stand-alone statistics
+    pass and the row counts leave partial 128- / 256-row tiles), the mode instead of a sample; then encode() of float
+    images (conv_in_tc) and the posterior sampled from its latent_dist."""
+    g = torch.Generator().manual_seed(56)
+    with audit_log.record("vae encoder ragged"):
+        vae_encoder.encode_video(_video(1, 3, 56, 128, 2).cuda(), sample=False)
+        x = torch.rand(2, 3, 56, 128, generator=g) * 2 - 1
+        dist = vae_encoder.encode(x.cuda()).latent_dist
+        dist.sample(noise=torch.randn(2, 4, 7, 16, generator=g).cuda())
+    _finish(audit_log)
+
+
+@pytest.fixture(scope="module")
+def vae_x4():
+    from lavie_b200.vae import X4_BLOCK_OUT, VAEDecoder, vae_synthetic_state_dict
+    m = VAEDecoder.x4_upscaler()
+    m.load_state_dict(vae_synthetic_state_dict(seed=0, block_out_channels=X4_BLOCK_OUT), strict=True)
+    return m.to("cuda").eval()
+
+
+def _x4_run(m, log, name, Fr, h, w, seed):
+    lat = 0.08333 * torch.randn(1, 4, Fr, h, w, generator=torch.Generator().manual_seed(seed))
+    with log.record(name):
+        m.decode_latents(lat.cuda())
+    _finish(log)
+
+
+@pytest.mark.gpu
+def test_audit_vae_x4(vae_x4, audit_log, reference_selfcheck):
+    """The VSR stage's decode: VSR-layout latents [1, 4, 2, 16, 24] (S = 384 tokens per frame in the wide attention)."""
+    _x4_run(vae_x4, audit_log, "vae x4", 2, 16, 24, 16)
+
+
+@pytest.mark.gpu
+def test_audit_vae_x4_ragged(vae_x4, audit_log, reference_selfcheck):
+    """2 frames of 12x22: S = 264, partial query and key tiles in attention_wide, M tails in the 128- / 256-channel
+    convs."""
+    _x4_run(vae_x4, audit_log, "vae x4 ragged", 2, 12, 22, 12)
+
+
+@pytest.mark.gpu
+@pytest.mark.skipif(os.environ.get("LAVIE_AUDIT_FULL") != "1", reason="full-geometry x4 audit: set LAVIE_AUDIT_FULL=1")
+def test_audit_vae_x4_full_frame(vae_x4, audit_log, reference_selfcheck):
+    """One frame of the VSR output geometry: a 320x512 latent decoded to 1280x2048, S = 163 840 (attention on the rows
+    of wide_query_rows).  Gated: minutes of fp64 references."""
+    _x4_run(vae_x4, audit_log, "vae x4 full frame", 1, 320, 512, 320)
+    print("\nper-launch audit (" + ", ".join(audit_log.runs) + ")\n" + audit_log.summary())
+
+
 @pytest.mark.gpu
 def test_coverage_ledger_and_summary(audit_log):
-    """Every launching function of ops was audited by the runs above or is named with the test that covers it; prints
-    the per-op summary (run with -s)."""
+    """Every launching function of every launch module was audited by the runs above or is named with the test that
+    covers it; prints the per-op summary (run with -s)."""
     missing_runs = [r for r in RUNS_DEFAULT if r not in audit_log.runs]
     if missing_runs:
         pytest.skip(f"the ledger needs every default audit run; not run: {missing_runs}")
     print("\nper-launch audit (" + ", ".join(audit_log.runs) + ")\n" + audit_log.summary())
-    names = launching_functions()
-    audited = {n for n, r in audit_log.rows.items() if r.launches}
-    unclassified = sorted(n for n in names if n not in audited and n not in COVERED_ELSEWHERE)
-    assert not unclassified, f"ops functions neither audited nor covered by a named test: {unclassified}"
+    audited = {key for key in CHECKERS if audit_log.rows[key[1]].launches}
+    unclassified = sorted(f"{m}.{n}" for m, n in launching_functions() if (m, n) not in audited
+                          and (m, n) not in COVERED_ELSEWHERE)
+    assert not unclassified, f"launching functions neither audited nor covered by a named test: {unclassified}"
     plans = set().union(*(audit_log.rows[n].plans for n in ("gemm", "conv3x3", "frame_conv")))
     assert "full-width" in plans and "main+tail window" in plans and any(p.startswith("split-K") for p in plans), plans
-    for n in ("attention", "frame_attention", "temporal_attention"):
+    assert "pad (0,1)" in audit_log.rows["conv3x3"].plans, audit_log.rows["conv3x3"].plans
+    for n in ("im2col_frames", "posterior_sample", "attention_wide"):
+        assert audit_log.rows[n].launches > 0, n
+    for n in PROBED:
         assert audit_log.rows[n].probes > 0, n
 
 
 # ------------------------------------------------------------------------------------------------ CPU: the ledger's list
 def test_ledger_classifies_every_launching_function():
+    assert {"ops", "vae_attention", "vae_encode_ops", "p2p", "check"} <= set(launch_modules())
     names = launching_functions()
-    assert {"gemm", "conv3x3", "attention", "pointwise_conv_nchw", "conv_in_tc", "groupnorm"} <= names
-    unknown = sorted(n for n in names if n not in CHECKERS and n not in COVERED_ELSEWHERE)
-    assert not unknown, f"new ops functions without a reference or a named covering test: {unknown}"
+    assert {("ops", n) for n in ("gemm", "conv3x3", "attention", "pointwise_conv_nchw", "conv_in_tc", "groupnorm")} <= names
+    unknown = sorted(f"{m}.{n}" for m, n in names if (m, n) not in CHECKERS and (m, n) not in COVERED_ELSEWHERE)
+    assert not unknown, f"launching functions without a reference or a named covering test: {unknown}"
+    stale = sorted(f"{m}.{n}" for m, n in list(CHECKERS) + list(COVERED_ELSEWHERE) if (m, n) not in names)
+    assert not stale, f"ledger entries that name no launching function: {stale}"
+    audited = [n for _, n in CHECKERS]
+    assert len(audited) == len(set(audited)), "the audit log keys its rows by function name"
+
+
+MODEL_SOURCES = MODEL_FILES + ("pipeline.py",)
+
+
+def test_model_code_calls_launches_through_the_module():
+    """The recorder replaces module attributes, so a launching function imported by name into a model file would run
+    unaudited: no model file may import one (`from .ops import gemm`, `from lavie_b200.vae_attention import ...`)."""
+    launching = collections.defaultdict(set)
+    for m, n in launching_functions():
+        launching[m].add(n)
+    bad = []
+    for fn in MODEL_SOURCES:
+        with open(os.path.join(PKG, fn)) as f:
+            tree = ast.parse(f.read(), fn)
+        for node in ast.walk(tree):
+            if not isinstance(node, ast.ImportFrom):
+                continue
+            mod = node.module or ""
+            if node.level == 0:
+                if not mod.startswith("lavie_b200."):
+                    continue
+                mod = mod[len("lavie_b200."):]
+            elif node.level != 1:
+                continue
+            bad += [f"{fn}:{node.lineno} imports {mod}.{al.name}" for al in node.names if al.name in launching.get(mod, ())]
+    assert not bad, bad
 
 
 def _fma32(a, b, c):
@@ -1557,3 +1897,123 @@ def test_upsample_phase_reference_is_nearest_upsample_then_conv():
     up = F.interpolate(x.to(F64).reshape(NF, H, W, C).permute(0, 3, 1, 2), scale_factor=2, mode="nearest")
     ref = F.conv2d(up, w, padding=1).permute(0, 2, 3, 1).reshape(-1, N)
     assert rel_l2(got, ref) < 1e-6                 # the packed phase taps are summed in fp32
+
+
+def test_padded_conv_reference_and_comparator_flag_symmetric_padding(monkeypatch):
+    """Downsample2D's conv (stride 2, padding (0, 1)) has the output size of the pad-1 conv on an even H, so a reference
+    with the wrong padding would compare a window shifted by one pixel: the padded reference is F.pad + conv2d, and the
+    comparator flags a kernel that padded (1, 1).  Comparison blocks of a few output lines exercise the line bands."""
+    from lavie_b200 import ops
+    for n in range(1, 20):
+        for st in (1, 2):
+            for pad in ((1, 1), (0, 1)):
+                assert conv_out_size(n, st, pad) == ops.conv3x3_out_size(n, st, pad), (n, st, pad)
+    g = torch.Generator().manual_seed(8)
+    NF, H, W, C, N = 2, 6, 10, 16, 24
+    x = torch.randn(NF * H * W, C, generator=g).to(BF16)
+    w = (torch.randn(N, 9 * C, generator=g) * (9 * C) ** -0.5).to(BF16)
+    acc, _ = conv_mm(x, NF, H, W, 2, w, (0, 1))
+    x4 = F.pad(x.to(F64).reshape(NF, H, W, C).permute(0, 3, 1, 2), (0, 1, 0, 1))
+    w4 = w.to(F64).reshape(N, 3, 3, C).permute(0, 3, 1, 2)
+    ref = F.conv2d(x4, w4, stride=2).permute(0, 2, 3, 1).reshape(-1, N)
+    assert acc.shape == ref.shape == (NF * 3 * 5, N) and rel_l2(acc, ref) < 1e-12
+    a = {"x": x, "NF": NF, "H": H, "W": W, "stride": 2, "padding": (0, 1), "w": w}
+    monkeypatch.setattr(Cmp, "STEP", 2 * 5 * 9 * C)            # two output lines per block
+    assert chk_conv3x3(a, _bf16_result(acc), {})[0].ok
+    sym, _ = conv_mm(x, NF, H, W, 2, w, (1, 1))
+    assert sym.shape == acc.shape
+    cmp = chk_conv3x3(a, _bf16_result(sym), {})[0]
+    assert not cmp.ok and cmp.n_over > acc.numel() // 2
+
+
+def _im2col_frames_loops(frames, kpad):
+    """The patch rows written tap by tap from the kernel's contract."""
+    N, H, W, _ = frames.shape
+    x = ((frames.float() / 255 - 0.5) / 0.5).to(BF16)
+    xp = torch.zeros(N, H + 2, W + 2, 3, dtype=BF16)
+    xp[:, 1:-1, 1:-1] = x
+    col = torch.zeros(N, H, W, kpad, dtype=BF16)
+    for c in range(3):
+        for kh in range(3):
+            for kw in range(3):
+                col[..., c * 9 + kh * 3 + kw] = xp[:, kh:kh + H, kw:kw + W, c]
+    return col.reshape(N * H * W, kpad)
+
+
+def test_im2col_frames_comparator_flags_defects():
+    frames = torch.randint(0, 256, (2, 5, 7, 3), dtype=torch.uint8, generator=torch.Generator().manual_seed(9))
+    frames[0, 0, 0] = torch.tensor([0, 255, 128], dtype=torch.uint8)
+    frames[1, 2, 3] = 127                   # the value a reciprocal-multiply normalisation rounds to another bf16
+    assert float(frame_values()[127]) == -0.003936767578125
+    a = {"frames": frames, "kpad": 32}
+    good = _im2col_frames_loops(frames, 32)
+    assert chk_im2col_frames(a, good, {})[0].ok
+    # pixel (0, 0) of frame 1: its kh = 0 taps read above the image and must stay zero
+    bad = good.clone()
+    bad[35, 9 + 1] = 0.5
+    cmp = chk_im2col_frames(a, bad, {})[0]
+    assert not cmp.ok and cmp.n_over == 1 and cmp.worst_at == (1, 0, 0, 10)
+    # one pad column (K index 27) written
+    bad = good.clone()
+    bad[12, 27] = 2.0 ** -8
+    cmp = chk_im2col_frames(a, bad, {})[0]
+    assert not cmp.ok and cmp.n_over == 1 and cmp.worst_at[-1] == 27
+
+
+def test_posterior_comparator_flags_defects():
+    B, Fr, h, w, scale = 2, 3, 4, 5, 0.18215
+    g = torch.Generator().manual_seed(10)
+    m = torch.randn(B * Fr, 8, h, w, generator=g)
+    m[:, 4:] *= 12.0
+    m[0, 4, 0, :4] = torch.tensor([-50.0, -30.0, 20.0, 45.0])
+    noise = torch.randn(B * Fr, 4, h, w, generator=g)
+
+    def kernel(lo=-30.0, hi=20.0, noise=noise):
+        z = m[:, :4] if noise is None else m[:, :4] + torch.exp(0.5 * m[:, 4:].clamp(lo, hi)) * noise
+        return (torch.tensor(scale, dtype=torch.float32) * z).reshape(B, Fr, 4, h, w).permute(0, 2, 1, 3, 4).contiguous()
+    a = {"moments": m, "B": B, "F": Fr, "scale": scale, "noise": noise}
+    assert chk_posterior_sample(a, kernel(), {})[0].ok
+    assert chk_posterior_sample(dict(a, noise=None), kernel(noise=None), {})[0].ok
+    assert not chk_posterior_sample(a, kernel(hi=21.0), {})[0].ok                   # logvar clamped at the wrong limit
+    frames_major = kernel().permute(0, 2, 1, 3, 4).reshape(B, 4, Fr, h, w)      # [B, F, 4, h, w] order in the output
+    assert not chk_posterior_sample(a, frames_major, {})[0].ok
+    assert not chk_posterior_sample(dict(a, noise=None), kernel(noise=None).transpose(0, 2).reshape(B, 4, Fr, h, w),
+                                    {})[0].ok
+
+
+def _fake_attention_wide(defect=None):
+    """A CPU stand-in for vae_attention.attention_wide: an honest kernel's bf16 output, or one that drops the last key
+    or the last 64-key tile of every frame."""
+    def run(q, k, v, frames, S, out=None):
+        o = torch.empty(frames, S, WIDE_D, dtype=F64)
+        keep = S - (1 if defect == "key" else (S - (S - 1) // 64 * 64) if defect == "tile" else 0)
+        for f in range(frames):
+            sl = slice(f * S, f * S + keep)
+            qq = q[f * S:(f + 1) * S].to(F64)
+            o[f] = torch.softmax(qq @ k[sl].to(F64).T, -1) @ v[sl].to(F64)
+        return _bf16_result(o.reshape(frames * S, WIDE_D))
+    return run
+
+
+def test_wide_attention_comparator_and_ramp_probe_flag_dropped_keys(monkeypatch):
+    """Self-similar q ~ k (each query attends to its own key) make the last key, or the last partial key tile, decide
+    the last query rows of every frame: the sampled-row comparator (which keeps the last query tile) and the key-ramp
+    probe both flag a kernel that drops them.  S = 1000: partial 128-query and 64-key tiles; the sampling threshold is
+    lowered so that the sampled path runs."""
+    monkeypatch.setitem(globals(), "WIDE_FULL_S", 256)
+    frames, S = 2, 1000
+    rows = wide_query_rows(S)
+    assert rows is not None and {0, 127, 896, 999} <= set(rows.tolist()) and len(rows) < S // 2
+    g = torch.Generator().manual_seed(11)
+    x = torch.randn(frames * S, WIDE_D, generator=g)
+    q, k, v = (0.1 * x).to(BF16), x.to(BF16), torch.randn(frames * S, WIDE_D, generator=g).to(BF16)
+    a = {"q": q, "k": k, "v": v, "frames": frames, "S": S, "out": None}
+    good = chk_attention_wide(a, _fake_attention_wide()(q, k, v, frames, S), {})
+    assert good[0].ok and "sampled" in good[0].what
+    assert all(c.ok for c in wide_attention_probes(_fake_attention_wide(), a))
+    for defect in ("key", "tile"):
+        fake = _fake_attention_wide(defect)
+        cmp = chk_attention_wide(a, fake(q, k, v, frames, S), {})[0]
+        assert not cmp.ok and cmp.worst_at[1] >= 960, (defect, str(cmp))
+        ones, ramp = wide_attention_probes(fake, a)
+        assert ones.ok and not ramp.ok, defect      # renormalised over the kept keys, V = 1 still gives 1

@@ -185,16 +185,14 @@ def test_posterior_sample_vs_fp64(with_noise):
     noise = torch.randn(B * Fr, 4, h, w, generator=torch.Generator().manual_seed(4)) if with_noise else None
     scale = 0.18215
     out = posterior_sample(m.to(DEV), B, Fr, scale, None if noise is None else noise.to(DEV)).cpu()
-    mean, lv = m[:, :4].to(F64), m[:, 4:].to(F64)
+    lv = m[:, 4:].to(F64)
     assert float(lv.min()) < -30 and float(lv.max()) > 20
     if noise is None:
         want = (m[:, :4] * scale).reshape(B, Fr, 4, h, w).permute(0, 2, 1, 3, 4)
         assert torch.equal(out, want)                    # the mode: one fp32 product per element
         return
-    std = torch.exp(0.5 * lv.clamp(-30, 20))
-    ref = scale * (mean + std * noise.to(F64))
-    bnd = 2.0 ** -20 * scale * (mean.abs() + std * noise.abs().to(F64)) + 1e-30
-    ref, bnd = (t.reshape(B, Fr, 4, h, w).permute(0, 2, 1, 3, 4) for t in (ref, bnd))
+    from test_launch_audit import posterior_ref               # the bound the per-launch audit holds the kernel to
+    ref, bnd = posterior_ref(m, B, Fr, scale, noise)
     assert bool(((out.to(F64) - ref).abs() <= bnd).all())
 
 
