@@ -269,19 +269,34 @@ def test_attention(batch, Sq, Sk, d, pitch, div):
     assert rel_l2(out.float(), ref) < 1e-2          # P is rounded to bf16 before P V
 
 
-@pytest.mark.parametrize("batch,Sq,Sk,d,pitch,div", [
-    (4, 200, 77, 40, 48, 2), (32, 2560, 77, 40, 48, 16), (8, 640, 77, 80, 80, 4), (4, 37, 20, 160, 160, 4),
-    (2, 16, 80, 64, 64, 1), (6, 100, 1, 128, 128, 3), (4, 5, 33, 96, 96, 2)])
-def test_short_key_attention_single_pass_kernel(batch, Sq, Sk, d, pitch, div):
+_SHORT_KEY_SHAPES = [(4, 200, 77, 40, 48, 2), (32, 2560, 77, 40, 48, 16), (8, 640, 77, 80, 80, 4), (4, 37, 20, 160, 160, 4),
+                     (2, 16, 80, 64, 64, 1), (6, 100, 1, 128, 128, 3), (4, 5, 33, 96, 96, 2)]
+
+
+@pytest.mark.parametrize("batch,Sq,Sk,d,pitch,div,inputs",
+                         [pytest.param(*s, "randn", id="-".join(map(str, s))) for s in _SHORT_KEY_SHAPES]
+                         + [pytest.param(*s, kind, id=f"{kind}-" + "-".join(map(str, s)))
+                            for kind in ("sharpened", "flush") for s in _SHORT_KEY_SHAPES])
+def test_short_key_attention_single_pass_kernel(batch, Sq, Sk, d, pitch, div, inputs):
     """The optional single-pass mma.sync kernel for Sk <= 80 (lavie_debug_set(8, 1); off by default -- it is bound by the
     legacy HMMA rate and not faster): same results as the tcgen05 flash kernel and as the fp32 reference, incl. ragged
-    query tiles, 1 key, every head dim."""
+    query tiles, 1 key, every head dim.  inputs: N(0, 1), or test_attention_rescale's sharpened (q x 16) and flush (the
+    keys from 64 on lifted by 130 log2 units) scores, which move the flash kernel's lazy maximum."""
     ops = _ops()
     from lavie_b200 import _lib
     lib = _lib.load()
     heads = 8
     q = _padded(batch * Sq, heads, d, pitch, 1)
     k = _padded(batch // div * Sk, heads, d, pitch, 2)
+    if inputs != "randn":
+        from test_attention_rescale import sharpen_heads
+        qh, kh = (t.reshape(t.shape[0], heads, pitch).float() for t in (q, k))
+        qh = qh.reshape(batch, Sq, heads, pitch).transpose(1, 2)
+        kh = kh.reshape(batch // div, Sk, heads, pitch).transpose(1, 2)
+        qs, ks = sharpen_heads(qh[..., :d], kh[..., :d], inputs, d ** -0.5)
+        qh[..., :d], kh[..., :d] = qs, ks
+        q = _bf(qh.transpose(1, 2).reshape(batch * Sq, heads * pitch))
+        k = _bf(kh.transpose(1, 2).reshape(batch // div * Sk, heads * pitch))
     v = _padded(batch // div * Sk, heads, d, pitch, 3)
     old = ops.attention(q, k, v, batch, heads, Sq, Sk, d, pitch, div)          # default: the tcgen05 flash kernel
     ref = _attn_ref(q, k, v, batch, heads, Sq, Sk, d, pitch, div)

@@ -361,6 +361,118 @@ def attention_core(Q, K, V, scale, bias=None, causal=False, rho=RHO_F32, c_p=C_A
     return o, bnd
 
 
+# ------------------------------------------------------------------------------------------------ lazy softmax rescale
+# The tcgen05 flash kernels (attn_fwd_kernel, attn_wide_kernel) walk the keys in 64-key tiles, one query row per thread
+# and 32 rows per warp.  The exponent offset m_used baked into O and the row sum l moves only when a tile's maximum, in
+# log2 units (fp32 max s times the fp32 scale_log2), exceeds m_used + 8; then O and l are multiplied by
+# alpha = 2^(m_used - m_tile), and the lanes of that warp that did not grow multiply by 1.
+LOG2E = 1.4426950408889634
+ATT_TILE = 64
+ATT_WARP = 32
+LAZY_THRESHOLD = 8.0
+Rescale = collections.namedtuple("Rescale", "events mixed first")
+
+
+def scale_log2(scale):
+    """The kernels' exponent scale: fp32(scale) * 1.4426950408889634f, rounded to fp32."""
+    return torch.tensor(scale, dtype=torch.float32) * torch.tensor(LOG2E, dtype=torch.float32)
+
+
+def key_tiles(keys, segments=1):
+    """(lo, hi) key ranges of the kernels' tile walk: `segments` equal key segments (SparseCausal: 2) of ceil(len / 64)
+    tiles each, the last tile of a segment possibly partial."""
+    n = keys // segments
+    return [(s * n + t, s * n + min(t + ATT_TILE, n)) for s in range(segments) for t in range(0, n, ATT_TILE)]
+
+
+def _warp_any(mask, rows):
+    """Per row: whether any real row of its 32-row warp is set (mask [..., rows])."""
+    pad = (-rows) % ATT_WARP
+    w = torch.cat([mask, mask.new_zeros(*mask.shape[:-1], pad)], -1)
+    w = w.reshape(*mask.shape[:-1], -1, ATT_WARP).any(-1, keepdim=True)
+    return w.expand(*w.shape[:-1], ATT_WARP).reshape(*mask.shape[:-1], rows + pad)[..., :rows]
+
+
+def tile_maxima(S, segments=1):
+    """fp32 maximum of every key tile (key_tiles) of scores S [..., rows, keys] -> [..., rows, tiles]."""
+    S = S.to(torch.float32)
+    n = S.shape[-1] // segments
+    pad = (-n) % ATT_TILE
+    segs = S.reshape(*S.shape[:-1], segments, n)
+    segs = torch.cat([segs, segs.new_full((*segs.shape[:-1], pad), -math.inf)], -1)
+    return segs.reshape(*S.shape[:-1], -1, ATT_TILE).amax(-1)
+
+
+def rescale_events(S, scale, segments=1, maxima=None):
+    """The kernels' lazy-maximum walk over fp32 scores S [..., rows, keys] (rows = queries of one sequence, in order), or
+    over their tile maxima (tile_maxima) given instead.  Returns Rescale(events: (row, tile) pairs at tile j > 0 whose
+    maximum grew past m_used + 8, mixed: whether a warp had growing and non-growing rows at the same tile, first:
+    (index..., row, tile) of the first event or None)."""
+    M = tile_maxima(S, segments) if maxima is None else maxima
+    sc = scale_log2(scale).to(M.device)
+    rows = M.shape[-2]
+    m_used = torch.full(M.shape[:-1], -math.inf, dtype=torch.float32, device=M.device)
+    events, mixed, first = 0, False, None
+    for j in range(M.shape[-1]):
+        m_tile = M[..., j] * sc
+        grow = m_tile > m_used + LAZY_THRESHOLD
+        if j > 0:
+            n = int(grow.sum())
+            if n:
+                events += n
+                if first is None:
+                    at = torch.unravel_index(grow.reshape(-1).nonzero()[0, 0].cpu(), tuple(grow.shape))
+                    first = tuple(int(i) for i in at) + (j,)
+                mixed = mixed or bool((_warp_any(grow, rows) & _warp_any(~grow, rows)).any())
+        m_used = torch.where(grow, m_tile, m_used)
+    return Rescale(events, mixed, first)
+
+
+LAZY_DEFECTS = ("o", "l", "sign", "warp", "partial", "stale")
+
+
+def lazy_attention_emulation(Q, K, V, scale, defect=None, ones=False, segments=1):
+    """The flash kernels' algorithm on the CPU, [batch, heads, S, d] tensors of bf16 values: fp32 scores, the lazy maximum
+    of rescale_events, p = 2^(s scale_log2 - m_used) (one fp32 rounding, as the kernels' fmaf) rounded to bf16 for P V,
+    O accumulated in fp32, the row sum l in fp32 over the unrounded p -- or, ones=True, over the bf16 P, as the ones column
+    of V accumulates it -- and o = O / l rounded to bf16.  `defect` injects one error into the rescale: "o" O not
+    rescaled, "l" l not rescaled, "sign" alpha = 2^(m_tile - m_used), "warp" alpha applied to every lane of a warp once
+    any lane grows, "partial" the threshold skipped on partial tiles, "stale" m_used not moved after the first tile."""
+    assert defect in (None,) + LAZY_DEFECTS, defect
+    S = Q.to(torch.float32) @ K.to(torch.float32).transpose(-1, -2)
+    V32 = V.to(torch.float32)
+    sc = scale_log2(scale)
+    rows = S.shape[-2]
+    m_used = torch.full(S.shape[:-1], -math.inf, dtype=torch.float32)
+    l = torch.zeros(S.shape[:-1], dtype=torch.float32)
+    O = torch.zeros(S.shape[:-1] + (V.shape[-1],), dtype=torch.float32)
+    for j, (lo, hi) in enumerate(key_tiles(S.shape[-1], segments)):
+        s = S[..., lo:hi]
+        m_tile = s.amax(-1) * sc
+        grow = m_tile > m_used + LAZY_THRESHOLD
+        if defect == "partial" and j > 0 and hi - lo < ATT_TILE:
+            grow = torch.zeros_like(grow)
+        if j > 0:
+            alpha = torch.where(grow, torch.exp2(m_used - m_tile), torch.ones_like(m_tile))
+            if defect == "sign":
+                alpha = torch.where(grow, torch.exp2(m_tile - m_used), torch.ones_like(m_tile))
+            elif defect == "warp":
+                alpha = torch.exp2(m_used - m_tile)
+            alpha = torch.where(_warp_any(grow, rows), alpha, torch.ones_like(alpha))
+            if defect != "o":
+                O = O * alpha[..., None]
+            if defect != ("o" if ones else "l"):     # the ones column is a column of O
+                l = l * alpha
+        if defect != "stale" or j == 0:
+            m_used = torch.where(grow, m_tile, m_used)
+        x = (s.to(F64) * sc.to(F64) - m_used.to(F64)[..., None]).to(torch.float32)
+        p = torch.exp2(x)
+        P = p.to(BF16).to(torch.float32)
+        l = l + (P if ones else p).sum(-1)
+        O = O + P @ V32[..., lo:hi, :]
+    return (O / l[..., None]).to(BF16)
+
+
 def rope64(t, table):
     """Rotate adjacent pairs (x0, x1) -> (x0 c - x1 s, x1 c + x0 s) of the first rot_pairs pairs; t [..., F, d],
     table [F, rot_pairs, 2] (cos, sin)."""
@@ -627,13 +739,20 @@ def attention_ref(a, v=None):
     return o, bnd
 
 
-def chk_attention(a, res, ctx):
+def attention_cmp(what, res, a, o, bnd):
+    """Cmp of an ops.attention result with the fp64 reference (o, bnd) of attention_ref, worst element located as
+    (batch, head, query, column)."""
     batch, heads, Sq, d = a["batch"], a["heads"], a["Sq"], a["d"]
-    o, bnd = attention_ref(a)
-    cmp = Cmp("attention", res, _attn_out(o, batch, heads, Sq, d), _attn_out(bnd, batch, heads, Sq, d), REL_ATTN)
+    cmp = Cmp(what, res, _attn_out(o, batch, heads, Sq, d), _attn_out(bnd, batch, heads, Sq, d), REL_ATTN)
     r, c = cmp.worst_at
     cmp.worst_at, cmp.dims = (r // Sq, c // d, r % Sq, c % d), ("batch", "head", "query", "column")
-    out = [cmp]
+    return cmp
+
+
+def chk_attention(a, res, ctx):
+    o, bnd = attention_ref(a)
+    out = [attention_cmp("attention", res, a, o, bnd)]
+    ctx["rescale_events"] = launch_events("attention", a).events
     if ctx.get("probe") is not None:
         out += ctx["probe"](a, res)
     return out
@@ -670,6 +789,7 @@ def _frame_cmp(what, res, o, bnd, a, rel_max):
 def chk_frame_attention(a, res, ctx):
     o, bnd = frame_attention_ref(a["qkv"], a["B"], a["F"], a["HW"], a["heads"], a["d"], a["head_pitch"])
     out = [_frame_cmp("frame attention", res, o, bnd, a, REL_ATTN)]
+    ctx["rescale_events"] = launch_events("frame_attention", a).events
     if ctx.get("probe") is not None:
         out += ctx["probe"](a, res)
     return out
@@ -945,6 +1065,7 @@ def chk_attention_wide(a, res, ctx):
     rows = wide_query_rows(a["S"])
     ref, bnd = wide_attention_ref(a["q"], a["k"], a["v"], a["frames"], a["S"], rows)
     out = [_wide_cmp("attention_wide" + (" (sampled rows)" if rows is not None else ""), res, a, rows, ref, bnd)]
+    ctx["rescale_events"] = launch_events("attention_wide", a).events
     if ctx.get("probe") is not None:
         out += ctx["probe"](a, res)
     return out
@@ -1056,7 +1177,8 @@ def attention_probes(name, real, a):
     """Launch the attention kernel `real` again on the recorded Q and K with probe values: V = 1 in every real head
     column (every output must be 1 within 2^-7: an extra or missing key or a wrong normalisation moves it by ~1/keys),
     then V = key-index ramps (ramp_values) in the first columns of every head, whose outputs must match the fp64
-    expected key index within the attention bound."""
+    expected key index within the attention bound; then the sharpened queries of sharpened_probe, which make the lazy
+    maximum move where the recorded scores may never."""
     if name == "attention_wide":
         return wide_attention_probes(real, a)
     heads, d, pitch = a["heads"], a["d"], a["head_pitch"]
@@ -1103,7 +1225,7 @@ def attention_probes(name, real, a):
         else:
             cols = (torch.arange(heads)[:, None] * d + torch.arange(ncol)).reshape(-1).to(got.device)
             out.append(Cmp(f"{name} probe V=key ramp", got[:, cols], ref[:, cols], bnd[:, cols]))
-    return out
+    return out + sharpened_probe(name, real, a)
 
 
 def wide_attention_probes(real, a):
@@ -1129,7 +1251,81 @@ def wide_attention_probes(real, a):
         else:
             ref, bnd = wide_attention_ref(q, k, v, frames, S, rows)
             out.append(_wide_cmp("attention_wide probe V=key ramp", got, a, rows, ref, bnd, cols=slice(0, 3)))
-    return out
+    return out + sharpened_probe("attention_wide", real, a)
+
+
+def _launch_heads(name, a):
+    """(Q, K, scale, segments) of an attention launch: per-head queries [n, heads, Sq, d] and the keys each query sequence
+    reads [n, heads, keys, d]."""
+    if name == "attention_wide":
+        frames, S = a["frames"], a["S"]
+        Q, K = (t.reshape(frames, 1, S, WIDE_D) for t in (a["q"], a["k"]))
+        return Q, K, 1.0, 1
+    heads, d, pitch = a["heads"], a["d"], a["head_pitch"]
+    if name == "frame_attention":
+        rows = frame_layout(a["B"], a["F"], a["HW"], a["qkv"].device)
+        hp = heads * pitch
+        return (heads_of(a["qkv"], rows, heads, pitch, d), heads_of(a["qkv"][:, hp:], rows, heads, pitch, d),
+                d ** -0.5, 1)
+    qrows, krows = attention_layout(a)
+    scale = a["scale"] if a["scale"] is not None else d ** -0.5
+    return (heads_of(a["q"], qrows, heads, pitch, d), heads_of(a["k"], krows, heads, pitch, d), scale,
+            2 if a["sparse_causal_frames"] else 1)
+
+
+def launch_events(name, a, q_mult=1.0):
+    """rescale_events of an attention launch (ops.attention, ops.frame_attention, attention_wide) with its queries times
+    q_mult (a power of two, so the fp32 scores scale exactly); the scores are formed in blocks of sequences and query
+    rows.  Launches of a single key tile cannot rescale: Rescale(0, False, None) without computing anything."""
+    Q, K, scale, segments = _launch_heads(name, a)
+    keys = K.shape[-2]
+    if segments == 1 and keys <= ATT_TILE:
+        return Rescale(0, False, None)
+    rows = max(128, (1 << 26) // max(1, Q.shape[1] * keys) // 128 * 128)
+    seqs = max(1, (1 << 26) // max(1, Q.shape[1] * Q.shape[2] * keys))
+    maxima = []
+    for lo in range(0, Q.shape[0], seqs):
+        k = K[lo:lo + seqs].to(torch.float32).transpose(-1, -2)
+        maxima.append(torch.cat([tile_maxima((Q[lo:lo + seqs, :, r0:r0 + rows].to(torch.float32) * q_mult) @ k, segments)
+                                 for r0 in range(0, Q.shape[2], rows)], -2))
+    return rescale_events(None, scale, maxima=torch.cat(maxima))
+
+
+def sharpened_probe(name, real, a):
+    """The launch again with its recorded queries times 2^s, s the smallest of 1..4 at which the lazy maximum moves at a
+    key tile j > 0 (launch_events), against the fp64 reference of the sharpened launch.  [] for launches of a single key
+    tile, for temporal attention (one whole-row maximum, no lazy path), and when no s up to 4 reaches an event.  The
+    comparison carries the events reached as `rescale_events`."""
+    if name == "temporal_attention":
+        return []
+    for s in range(1, 5):
+        ev = launch_events(name, a, 2.0 ** s)
+        if ev.events:
+            break
+    else:
+        return []
+    m = 2.0 ** s
+    what = f"{name} probe q x 2^{s}"
+    if name == "attention_wide":
+        rows = wide_query_rows(a["S"])
+        q = a["q"] * m
+        got = real(q, a["k"], a["v"], a["frames"], a["S"])
+        ref, bnd = wide_attention_ref(q, a["k"], a["v"], a["frames"], a["S"], rows)
+        cmp = _wide_cmp(what, got, a, rows, ref, bnd)
+    elif name == "frame_attention":
+        qkv = a["qkv"].clone()
+        qkv[:, :a["heads"] * a["head_pitch"]] *= m
+        got = real(qkv, a["B"], a["F"], a["HW"], a["heads"], a["d"], a["head_pitch"])
+        o, bnd = frame_attention_ref(qkv, a["B"], a["F"], a["HW"], a["heads"], a["d"], a["head_pitch"])
+        cmp = _frame_cmp(what, got, o, bnd, a, REL_ATTN)
+    else:
+        sa = dict(a, q=a["q"] * m)
+        got = real(sa["q"], a["k"], a["v"], a["batch"], a["heads"], a["Sq"], a["Sk"], a["d"], a["head_pitch"],
+                   a["kv_batch_div"], a["scale"], None, a["sparse_causal_frames"], a["sc_halo"])
+        o, bnd = attention_ref(sa)
+        cmp = attention_cmp(what, got, sa, o, bnd)
+    cmp.rescale_events = ev.events
+    return [cmp]
 
 
 # ------------------------------------------------------------------------------------------------ recorder
@@ -1181,6 +1377,8 @@ class OpRow:
         self.worst_rel = 0.0
         self.plans = set()
         self.probes = 0
+        self.events = 0           # lazy-maximum rescales (rescale_events) the recorded launches reach
+        self.probe_events = 0     # ... and the sharpened probes
 
 
 class Recorder:
@@ -1271,7 +1469,7 @@ class Recorder:
                 geom = None
             for r in results:
                 decode_item_frame(r, geom, res.shape[0] if res.dim() == 2 else -1)
-            self._record(name, idx, block, a, results, plans, "probe" in ctx)
+            self._record(name, idx, block, a, results, plans, "probe" in ctx, ctx.get("rescale_events", 0))
             return res
 
         wrapper.__wrapped__ = fn
@@ -1280,11 +1478,13 @@ class Recorder:
     def _probe(self, name, a, res):
         return attention_probes(name, self.real[name][1], a)
 
-    def _record(self, name, idx, block, a, results, plans, probed):
+    def _record(self, name, idx, block, a, results, plans, probed, events=0):
         row = self.log.rows[name]
         row.launches += 1
         row.plans |= plans
         row.probes += int(probed)
+        row.events += events
+        row.probe_events += sum(getattr(r, "rescale_events", 0) for r in results)
         for r in results:
             row.worst = max(row.worst, r.worst)
             row.worst_rel = max(row.worst_rel, r.rel if isinstance(r, Cmp) else 0.0)
@@ -1308,10 +1508,13 @@ class AuditLog:
         return Recorder(self)
 
     def summary(self):
-        lines = [f"{'op':24s} {'launches':>8s} {'probes':>6s} {'worst err/bound':>15s} {'worst rel-L2':>12s}  plans"]
+        # rescales: lazy-maximum moves at key tiles j > 0 (rescale_events), in the recorded launches / in the probes
+        lines = [f"{'op':24s} {'launches':>8s} {'probes':>6s} {'worst err/bound':>15s} {'worst rel-L2':>12s} "
+                 f"{'rescales rec/probe':>18s}  plans"]
         for name in sorted(self.rows):
             r = self.rows[name]
-            lines.append(f"{name:24s} {r.launches:8d} {r.probes:6d} {r.worst:15.3g} {r.worst_rel:12.3g}  "
+            ev = f"{r.events}/{r.probe_events}" if name in PROBED else "-"
+            lines.append(f"{name:24s} {r.launches:8d} {r.probes:6d} {r.worst:15.3g} {r.worst_rel:12.3g} {ev:>18s}  "
                          f"{', '.join(sorted(r.plans))}")
         return "\n".join(lines)
 
@@ -1765,6 +1968,21 @@ def _fake_attention(defect=None):
     return run
 
 
+def _lazy_fake_attention(defect=None):
+    """A CPU stand-in for ops.attention running the kernels' lazy-rescale algorithm (lazy_attention_emulation), with
+    the ones-column denominator when d % 16 != 0, honest or with one rescale defect."""
+    def run(q, k, v, batch, heads, Sq, Sk, d, pitch, kv_batch_div=1, scale=None, out=None, sparse_causal_frames=0,
+            sc_halo=0):
+        a = {"q": q, "k": k, "v": v, "batch": batch, "heads": heads, "Sq": Sq, "Sk": Sk, "d": d, "head_pitch": pitch,
+             "kv_batch_div": kv_batch_div, "sparse_causal_frames": sparse_causal_frames, "sc_halo": sc_halo}
+        qrows, krows = attention_layout(a)
+        Q, K, V = (heads_of(t, r, heads, pitch, d) for t, r in ((q, qrows), (k, krows), (v, krows)))
+        o = lazy_attention_emulation(Q, K, V, d ** -0.5 if scale is None else scale, defect, ones=d % 16 != 0,
+                                     segments=2 if sparse_causal_frames else 1)
+        return _attn_out(o, batch, heads, Sq, d)
+    return run
+
+
 def _attn_args(batch=4, heads=2, Sq=9, Sk=20, d=16, pitch=16, div=2, seed=0):
     g = torch.Generator().manual_seed(seed)
     q = torch.randn(batch * Sq, heads * pitch, generator=g).to(BF16)
@@ -1784,6 +2002,19 @@ def test_attention_probes_flag_key_mask_defects():
     assert not ones.ok                      # one extra zero-score, zero-value key
     ones, ramp = attention_probes("attention", _fake_attention("drop"), a)
     assert not (ones.ok and ramp.ok)        # the last key dropped
+    # the lazy rescale: 150 keys (two full tiles and a partial one), N(0, 1) scores that never move the maximum; the
+    # sharpened probe (q x 2^s) does, and flags each rescale defect of the kernels' algorithm
+    # (d = 40: the ones column carries the row sum through O, so the separate l is not used; skipping the threshold on a
+    # partial tile only shifts the exponent offset, which matters once p overflows -- test_attention_rescale.py's
+    # spike and flush inputs)
+    for d, pitch, flagged in ((48, 48, ("o", "l", "sign", "warp", "stale")), (40, 48, ("o", "sign", "warp", "stale"))):
+        a = _attn_args(Sq=40, Sk=150, d=d, pitch=pitch)
+        assert launch_events("attention", a).events == 0
+        probes = attention_probes("attention", _lazy_fake_attention(), a)
+        assert len(probes) == 3 and all(c.ok for c in probes) and probes[2].rescale_events > 0, [str(c) for c in probes]
+        for defect in LAZY_DEFECTS:
+            sharp = attention_probes("attention", _lazy_fake_attention(defect), a)[2]
+            assert sharp.ok != (defect in flagged), (d, defect, str(sharp))
 
 
 def test_key_ramp_tells_adjacent_keys_apart_at_long_sequences():
@@ -2015,5 +2246,5 @@ def test_wide_attention_comparator_and_ramp_probe_flag_dropped_keys(monkeypatch)
         fake = _fake_attention_wide(defect)
         cmp = chk_attention_wide(a, fake(q, k, v, frames, S), {})[0]
         assert not cmp.ok and cmp.worst_at[1] >= 960, (defect, str(cmp))
-        ones, ramp = wide_attention_probes(fake, a)
+        ones, ramp = wide_attention_probes(fake, a)[:2]
         assert ones.ok and not ramp.ok, defect      # renormalised over the kept keys, V = 1 still gives 1
