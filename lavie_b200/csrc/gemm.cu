@@ -560,7 +560,7 @@ gemm_bf16_tcgen05(const __grid_constant__ CUtensorMap tmap_a0, const __grid_cons
           float f[32];
 #pragma unroll
           for (int e = 0; e < 32; ++e) f[e] = __uint_as_float(v[e]);
-          if (col0 < p.N) {
+          if (col0 + 32 <= p.N) {
             if (p.bias) {                          // warp-uniform addresses: broadcast loads
 #pragma unroll
               for (int e = 0; e < 32; e += 4) {
@@ -573,6 +573,23 @@ gemm_bf16_tcgen05(const __grid_constant__ CUtensorMap tmap_a0, const __grid_cons
               for (int e = 0; e < 32; e += 4) {
                 const float4 b4 = __ldg(reinterpret_cast<const float4*>(rb_row + col0 + e));
                 f[e] += b4.x; f[e + 1] += b4.y; f[e + 2] += b4.z; f[e + 3] += b4.w;
+              }
+            }
+          } else if (col0 < p.N) {
+            // the last chunk of an N % 32 != 0 output: its columns past N are clipped by the TMA store, and their bias
+            // loads must not read past the caller's [N] rows (N % 8 == 0: whole float4s).  A separate branch so that
+            // the full chunks keep their unpredicated loads (the guard in every chunk measured ~2% slower per step)
+#pragma unroll
+            for (int e = 0; e < 32; e += 4) {
+              if (col0 + e < p.N) {
+                if (p.bias) {
+                  const float4 b4 = __ldg(reinterpret_cast<const float4*>(p.bias + col0 + e));
+                  f[e] += b4.x; f[e + 1] += b4.y; f[e + 2] += b4.z; f[e + 3] += b4.w;
+                }
+                if (rb_row) {
+                  const float4 b4 = __ldg(reinterpret_cast<const float4*>(rb_row + col0 + e));
+                  f[e] += b4.x; f[e + 1] += b4.y; f[e + 2] += b4.z; f[e + 3] += b4.w;
+                }
               }
             }
           }
@@ -922,8 +939,9 @@ int g_debug = 0;
 int g_k_rot = 0;   // measured: no effect on B200 (profiles/r1_notes.md), kept as a tuning hook only
 int g_no_tail = 0; // lavie_debug_set(5, 1): never split a GEMM into main + tail launches (A/B timing)
 int g_inkernel_reduce = 0;   // lavie_debug_set(7, 1): the last-arriving CTA of a block sums the split-K planes in the kernel
-                             // instead of the separate reduction kernel.  Correct (same bits), but measured SLOWER on the
-                             // full step (profiles/r2_ab_inkernel_splitk.txt): off by default, kept for A/B.
+                             // instead of the separate reduction kernel.  Correct (same output bits; the column statistics
+                             // are summed in the epilogue's order, so they differ in the last fp32 bits), but measured
+                             // SLOWER on the full step (profiles/r2_ab_inkernel_splitk.txt): off by default, kept for A/B.
 constexpr size_t TICKET_BYTES = 64 * 1024;   // tail of the caller's workspace: zero before first use, left zero
 int num_sms() { return lavie_num_sms(); }
 

@@ -81,13 +81,25 @@ def test_gemm_wide_tile_epilogue(N):
     assert rel_l2(out.float(), ref) < 4e-3
 
 
+def _plan(M, N, K, conv=0):
+    """(bn, splits, tail_tiles, tail_splits) of the library's planner for the split-K workspace ops passes."""
+    import ctypes
+    from lavie_b200 import _lib
+    bn, s, tail, ts = (ctypes.c_int() for _ in range(4))
+    assert _lib.load().lavie_gemm_plan(M, N, K, conv, 0, _ops().WORKSPACE_BYTES, bn, s, tail, ts) == 0
+    return bn.value, s.value, tail.value, ts.value
+
+
 def test_gemm_main_plus_splitk_tail_window():
     """More than one wave of tiles with a nearly empty last wave: the planner issues full waves over the leading tile
     rows and a split-K launch over the rest.  Same epilogue on both paths; compare with the single-launch result."""
     ops = _ops()
     from lavie_b200 import _lib
     lib = _lib.load()
-    M, N, K, B = 256 * 39 + 100, 640, 2048, 2
+    M, N, K, B = 256 * 74 + 100, 640, 2048, 2
+    bn, s, tail, ts = _plan(M, N, K)
+    assert s == 1 and tail > 0 and ts > 1, (bn, s, tail, ts)      # the shape must keep planning a split-K tail window
+    main_rows = ((M + 255) // 256 - tail) * 256
     a = _bf(_rand(M, K))
     w = _bf(_rand(N, K, scale=K ** -0.5))
     bias = _rand(N, seed=1)
@@ -97,19 +109,22 @@ def test_gemm_main_plus_splitk_tail_window():
     out = ops.gemm(a, w, bias=bias, row_bias=rb, rows_per_batch=rpb, residual=res)
     lib.lavie_debug_set(5, 1)
     try:
+        assert _plan(M, N, K)[1:3] == (1, 0)
         single = ops.gemm(a, w, bias=bias, row_bias=rb, rows_per_batch=rpb, residual=res)
     finally:
         lib.lavie_debug_set(5, 0)
     ref = a.float() @ w.float().t() + bias + rb.repeat_interleave(rpb, 0)[:M] + res.float()
     assert rel_l2(out.float(), ref) < 4e-3
     assert rel_l2(out.float(), single.float()) < 3e-3     # split-K changes the summation order of the tail rows only
-    assert torch.equal(out[: 256 * 30], single[: 256 * 30])
+    assert torch.equal(out[:main_rows], single[:main_rows])
 
 
 def test_conv3x3_main_plus_tail_window():
     ops = _ops()
     from lavie_b200.packing import pack_conv3x3
-    NF, H, W, C, N = 32, 10, 16, 128, 1280
+    NF, H, W, C, N = 29, 10, 16, 512, 1280
+    bn, s, tail, ts = _plan(NF * H * W, N, 9 * C, conv=1)
+    assert s == 1 and tail > 0 and ts > 1, (bn, s, tail, ts)      # the shape must keep planning a split-K tail window
     x = _bf(_rand(NF * H * W, C))
     w = _bf(_rand(N, C, 3, 3, scale=(9 * C) ** -0.5))
     res = _bf(_rand(NF * H * W, N, seed=5))

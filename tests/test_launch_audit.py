@@ -1413,11 +1413,11 @@ class Recorder:
         bn, sp, tt, ts = (ctypes.c_int() for _ in range(4))
         self.lib.lavie_gemm_plan(M, N, K, conv, int(geglu), self.ops.WORKSPACE_BYTES, ctypes.byref(bn), ctypes.byref(sp),
                                  ctypes.byref(tt), ctypes.byref(ts))
-        kinds = set()
-        kinds.add(f"split-K x{sp.value}" if sp.value > 1 else "full-width")
         if tt.value:
-            kinds.add("main+tail window")
-        return kinds, max(sp.value, ts.value, 1)
+            kind = f"bn{bn.value} main+tail x{ts.value}"
+        else:
+            kind = f"bn{bn.value} split-K x{sp.value}" if sp.value > 1 else f"bn{bn.value} full-width"
+        return {kind}, max(sp.value, ts.value, 1)
 
     def _wrap(self, name, fn, check):
         sig = inspect.signature(fn)
@@ -1791,7 +1791,8 @@ def test_coverage_ledger_and_summary(audit_log):
                           and (m, n) not in COVERED_ELSEWHERE)
     assert not unclassified, f"launching functions neither audited nor covered by a named test: {unclassified}"
     plans = set().union(*(audit_log.rows[n].plans for n in ("gemm", "conv3x3", "frame_conv")))
-    assert "full-width" in plans and "main+tail window" in plans and any(p.startswith("split-K") for p in plans), plans
+    for kind in ("full-width", "main+tail", "split-K"):
+        assert any(kind in p for p in plans), (kind, plans)
     assert "pad (0,1)" in audit_log.rows["conv3x3"].plans, audit_log.rows["conv3x3"].plans
     for n in ("im2col_frames", "posterior_sample", "attention_wide"):
         assert audit_log.rows[n].launches > 0, n
